@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- encode/decode GSamples/s of the FLAC hot path on B200 (driver contract).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c3|c5|c4]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c3|c5|c4] [--dump-outputs DIR]
 
 Workload (default c3 = BASELINE.json configs[2], the configuration the encode-scaling metric is
 quoted on; it fits one GPU): synthetic Sentinel-2-like 10980x10980 uint16, 8 bands, streaming
@@ -25,7 +25,11 @@ second labelled CPU row: FFmpeg libavcodec's FLAC encoder and decoder on one cor
 `e2e` is the same step through the public engine API with HOST (pinned) buffers: H2D of the
 raster and D2H of the frames inside the timed region.  "c5_bbox" is BASELINE.json configs[4]
 through the public API: SpatialFLACStreamer.get_tiles_by_bbox over a 4096-tile container, the
-requested tiles split over the ranks.
+requested tiles split over the ranks.  Every timed section runs K steps after its warm-up.
+
+`--dump-outputs DIR` writes what the last timed encode and decode steps returned as DIR/<name>.npy (float32 / float64,
+the frame bytes and the decoded raster as a fixed seeded sample of 2^22 elements each, under 64 MB in all); the inputs
+are synthetic and seeded, so two builds run with the same arguments can be compared array for array.
 
 `--impl reference` times the reference's CPU implementation of the path (the oracle port of
 libFLAC's procedure + the reference's numpy normalisation, one tile per task in a process pool over
@@ -387,7 +391,14 @@ def main():
     ap.add_argument("--cpu-tiles", type=int, default=0, help="tiles in the CPU baseline sample (0 = auto)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the weak-scaling, container and c5_bbox sections")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last encode and decode step returned as DIR/<name>.npy (float32/float64; "
+                         "payload bytes and raster pixels as a fixed seeded sample; rank 0's tiles when there are several ranks)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -484,6 +495,7 @@ def run_ours(args, rank, world, local):
     enc_ms = ev0.elapsed_time(ev1) / args.steps
     enc = state["enc"]
     comp_bytes = int(enc.sizes.sum())
+    dump = encode_outputs(enc) if args.dump_outputs and rank == 0 else None
 
     # ---- decode direction ------------------------------------------------------------------
     payload = torch.cat([enc.payload, torch.zeros(64, dtype=torch.uint8, device=dev)])
@@ -498,7 +510,7 @@ def run_ours(args, rank, world, local):
         return eng.decode_tiles(payload, enc.offsets, enc.sizes, tiles, enc.sample_rates, enc.minmax, scale, out, enc.bps, enc.blocksize,
                                 index=index)
 
-    for _ in range(args.warmup):
+    for _ in range(max(1, args.warmup)):           # at least one: its status and raster are checked below
         st = decode_step(None)
     assert list(st[:3]) == [0, 0, 0], f"decode status {st}"
     foreign_ok = all(bool(torch.equal(out[:, int(t["row_off"]):int(t["row_off"] + t["h"]), int(t["col_off"]):int(t["col_off"] + t["w"])],
@@ -514,7 +526,7 @@ def run_ours(args, rank, world, local):
     barrier()
     dec_foreign_ms = evf0.elapsed_time(evf1) / args.steps
     out.zero_()
-    for _ in range(args.warmup):
+    for _ in range(max(1, args.warmup)):
         st = decode_step()
     assert list(st[:3]) == [0, 0, 0], f"decode status {st}"
     if enc.bits_per_sample == 16:
@@ -536,12 +548,15 @@ def run_ours(args, rank, world, local):
     ev2, ev3 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev2.record()
     for _ in range(args.steps):
-        decode_step()
+        st = decode_step()
         prof(dec_prof, {"k_decode_subframes": 1})
     ev3.record()
     barrier()
     dec_launches = L.frb_launch_count() - dlaunch0
     dec_ms = ev2.elapsed_time(ev3) / args.steps
+    if dump is not None:
+        dump.update(decode_outputs(out, st))
+        write_outputs(args.dump_outputs, dump)
     clocks = sampler.stop() if rank == 0 else None
 
     # ---- e2e: host (pinned) raster in, host frames out -----------------------------------------
@@ -564,7 +579,7 @@ def run_ours(args, rank, world, local):
     t0 = time.perf_counter()
     ev4, ev5 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev4.record()
-    e2e_steps = max(1, min(args.steps, 3))
+    e2e_steps = args.steps
     for _ in range(e2e_steps):
         nout = e2e_step()
     ev5.record()
@@ -613,7 +628,7 @@ def run_ours(args, rank, world, local):
         barrier()
         evw0, evw1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         evw0.record()
-        wsteps = max(1, min(args.steps, 3))
+        wsteps = args.steps
         for _ in range(wsteps):
             eng.encode_tiles(full, tiles_full, level)
         evw1.record()
@@ -628,7 +643,7 @@ def run_ours(args, rank, world, local):
         eng.release()
         torch.cuda.empty_cache()
         try:
-            c5 = c5_bbox_sweep(eng, rank, world, dev, barrier)
+            c5 = c5_bbox_sweep(eng, rank, world, dev, barrier, reps=args.steps)
         except Exception as ex:  # noqa: BLE001
             c5 = {"error": repr(ex)}
 
@@ -755,6 +770,50 @@ def run_ours(args, rank, world, local):
 
 def raster_elem_size(workload: str) -> int:
     return 4 if workload == "c4" else 2
+
+
+# --dump-outputs: outputs larger than DUMP_SAMPLE elements (the frame bytes, the decoded raster) are kept as a sample at
+# positions drawn from a fixed seed, so that two builds can be compared output for output within DUMP_LIMIT bytes
+DUMP_SAMPLE = 1 << 22
+DUMP_LIMIT = 64 << 20
+
+
+def sample_positions(n_total: int, seed: int) -> np.ndarray:
+    if n_total <= DUMP_SAMPLE:
+        return np.arange(n_total, dtype=np.int64)
+    return np.sort(np.random.default_rng(seed).integers(0, n_total, DUMP_SAMPLE, dtype=np.int64))
+
+
+def encode_outputs(enc) -> dict:
+    """What Engine.encode_tiles returned (EncodedTiles): integers as float64 (exact), frame bytes sampled as float32."""
+    import torch
+    pos = torch.from_numpy(sample_positions(int(enc.payload.numel()), seed=1)).to(enc.payload.device)
+    res = {"encode_payload_sample": enc.payload[pos].cpu().numpy().astype(np.float32)}
+    for name in ("offsets", "sizes", "minmax", "n_samples", "sample_rates"):
+        res["encode_" + name] = np.asarray(getattr(enc, name), dtype=np.float64)
+    for name in ("frame_bytes", "sub_bitoff"):             # int32 views of uint32 data
+        res["encode_" + name] = getattr(enc, name).cpu().numpy().view(np.uint32).astype(np.float64)
+    return res
+
+
+def decode_outputs(out, status) -> dict:
+    """What Engine.decode_tiles produced: the raster it wrote (sampled; uint16, int16 and float32 are exact in float32) and
+    the status words it returned."""
+    import torch
+    flat = (out.view(torch.int16) if out.dtype == torch.uint16 else out).reshape(-1)
+    vals = flat[torch.from_numpy(sample_positions(flat.numel(), seed=2)).to(flat.device)].cpu().numpy()
+    if out.dtype == torch.uint16:
+        vals = vals.view(np.uint16)
+    return {"decode_raster_sample": vals.astype(np.float32), "decode_status": np.asarray(status, dtype=np.float64)}
+
+
+def write_outputs(directory: str, arrays: dict) -> None:
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT, f"--dump-outputs: {total} bytes exceed {DUMP_LIMIT}"
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+    print(f"[bench] wrote {len(arrays)} arrays ({total} bytes) to {directory}", file=sys.stderr)
 
 
 def _scratch_dir(rank, world, dev):

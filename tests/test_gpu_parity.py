@@ -334,17 +334,24 @@ def test_encode_golden_rgb_is_byte_identical_to_libflac(nat, rgb_pcm):
 
 
 def test_gpu_streams_accepted_by_ffmpeg(nat):
-    ff = pytest.importorskip("oracle.ffmpeg_flac")
-    if not ff.available():
-        pytest.skip("bundled FFmpeg libraries not found")
+    """FFmpeg libavcodec accepts the GPU's level-8 streams: every stream is byte for byte one that FFmpeg decoded to the
+    input samples (tests/golden/ffmpeg_decoded.json, made by make_ffmpeg_golden.py), and where the bundled FFmpeg
+    libraries are installed they decode it again."""
+    import hashlib
     from flac_raster_b200 import flacfmt
-    for name, (x, bps) in signal_cases().items():
-        if name == "tiny3":
-            continue
+    from oracle import ffmpeg_flac as ff
+    golden = json.loads((GOLDEN / "ffmpeg_decoded.json").read_text())["gpu_level8"]
+    live = ff.available()
+    cases = {k: v for k, v in signal_cases().items() if k != "tiny3"}        # FFmpeg refuses blocksize < 16
+    assert set(golden) == set(cases)
+    for name, (x, bps) in cases.items():
         payload, _ = nat.host_encode(x, bps, 48000, 8)
         si = flacfmt.StreamInfo(4096, 4096, 0, 0, 48000, x.shape[1], bps, x.shape[0])
-        out = ff.decode_bytes(flacfmt.build_header(si) + bytes(payload), x.shape[1])
-        assert np.array_equal(out, x), name
+        stream = flacfmt.build_header(si) + bytes(payload)
+        assert hashlib.md5(stream).hexdigest() == golden[name]["stream_md5"], name
+        assert hashlib.md5(np.ascontiguousarray(x, dtype="<i4").tobytes()).hexdigest() == golden[name]["decoded_md5"], name
+        if live:
+            assert np.array_equal(ff.decode_bytes(stream, x.shape[1]), x), name
 
 
 def test_pyflac_shim_callback_contract(nat, oracle, tmp_path):

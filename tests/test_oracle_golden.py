@@ -1,5 +1,6 @@
 """CPU suite part 1: the oracle is pinned against the reference's golden vectors (SURVEY.md 8c)."""
 import hashlib
+import json
 
 import numpy as np
 import pytest
@@ -91,16 +92,20 @@ def test_oracle_roundtrip_all_levels(oracle, level):
 
 
 def test_oracle_streams_accepted_by_ffmpeg(oracle):
-    """A second, unrelated production decoder (FFmpeg libavcodec) accepts the oracle's streams."""
-    ff = pytest.importorskip("oracle.ffmpeg_flac")
-    if not ff.available():
-        pytest.skip("bundled FFmpeg libraries not found")
-    for name, (x, bps) in signal_cases().items():
-        if name == "tiny3":
-            continue        # FFmpeg refuses blocksize < 16
+    """A second, unrelated production decoder (FFmpeg libavcodec) accepts the oracle's streams: every stream is byte for
+    byte one that FFmpeg decoded to the input samples (tests/golden/ffmpeg_decoded.json, made by make_ffmpeg_golden.py),
+    and where the bundled FFmpeg libraries are installed they decode it again."""
+    from oracle import ffmpeg_flac as ff
+    golden = json.loads((GOLDEN / "ffmpeg_decoded.json").read_text())["oracle_level5"]
+    live = ff.available()
+    cases = {k: v for k, v in signal_cases().items() if k != "tiny3"}        # FFmpeg refuses blocksize < 16
+    assert set(golden) == set(cases)
+    for name, (x, bps) in cases.items():
         enc, _ = oracle.encode(x, bps, 48000, 5, finalize=True)
-        out = ff.decode_bytes(enc, x.shape[1])
-        assert np.array_equal(out, x), name
+        assert hashlib.md5(enc).hexdigest() == golden[name]["stream_md5"], name
+        assert hashlib.md5(np.ascontiguousarray(x, dtype="<i4").tobytes()).hexdigest() == golden[name]["decoded_md5"], name
+        if live:
+            assert np.array_equal(ff.decode_bytes(enc, x.shape[1]), x), name
 
 
 def test_oracle_rejects_corruption(oracle):
