@@ -77,7 +77,9 @@ class StreamEncoder:
     def _init(self):
         if not (0 <= self._compression_level <= 8):
             self._compression_level = 8 if self._compression_level > 8 else 0
-        bs = self._blocksize or 4096
+        # blocksize 0 (pyflac's default) follows libFLAC's init_stream: 1152 for the presets without LPC (levels 0-2,
+        # max_lpc_order == 0), 4096 otherwise
+        bs = self._blocksize or (1152 if self._compression_level <= 2 else 4096)
         if not (16 <= bs <= 4096):
             raise EncoderInitException("FLAC__STREAM_ENCODER_INIT_STATUS_INVALID_BLOCK_SIZE")
         if not (1 <= self._channels <= 8):

@@ -234,13 +234,14 @@ extern "C" int frb_stream_encoder_init_stream(frb_stream_encoder *e, frb_encoder
     if (e->channels < 1 || e->channels > FRB_MAX_CHANNELS) return 4;
     if (e->bps != 16 && e->bps != 32) return 5;                 // what pyflac can ask for (docs/sonos-pyflac.txt:1988-1991)
     if (e->sample_rate == 0 || e->sample_rate > 1048575u) return 6;
-    if (e->blocksize == 0) e->blocksize = 4096;              // libFLAC picks 4096 for LPC presets
+    if (e->level > 8) e->level = 8;
+    // blocksize 0 (pyflac's default): libFLAC's init_stream picks 1152 when max_lpc_order == 0 (levels 0-2), 4096 otherwise
+    if (e->blocksize == 0) e->blocksize = e->level <= 2 ? 1152 : 4096;
     if (e->blocksize < 16 || e->blocksize > FRB_MAX_BLOCKSIZE) return 7;
     // streamable subset (format.h rules quoted at docs/sonos-pyflac.txt:3498, :3527): <= 48 kHz caps the blocksize at 4608 and the
     // LPC order at 12 -- every preset of this engine satisfies both, so the flag only has to be accepted.
     // limit_min_bitrate (forces at least one non-constant subframe per frame in libFLAC 1.4) is not implemented.
     if (e->limit_min_bitrate) return 1;
-    if (e->level > 8) e->level = 8;
     frb_encode_params p = {1, e->channels, e->bps, e->blocksize, e->level, 0};
     if (!frb::enc_params_ok(&p)) return 1;
     e->cb = write_cb; e->seek_cb = seek_cb; e->tell_cb = tell_cb; e->meta_cb = metadata_cb; e->client = client_data;
