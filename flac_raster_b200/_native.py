@@ -60,6 +60,12 @@ TILE_HEADER_DTYPE = np.dtype([
     ("data_min", "<f8"), ("data_max", "<f8"), ("nodata", "<f8"),
 ])
 
+# frb_window_stream: a run of frames [first_frame, first_frame + n_frames) of a stream of total_samples samples
+WINDOW_STREAM_DTYPE = np.dtype([
+    ("byte_offset", "<u8"), ("byte_length", "<u8"), ("total_samples", "<u8"), ("audio_base", "<i8"),
+    ("sample_rate", "<u4"), ("frame_base", "<u4"), ("first_frame", "<u4"), ("n_frames", "<u4"),
+])
+
 DECODE_STREAM_DTYPE = np.dtype([
     ("byte_offset", "<u8"), ("byte_length", "<u8"), ("n_samples", "<u8"), ("audio_base", "<i8"),
     ("sample_rate", "<u4"), ("frame_base", "<u4"),
@@ -93,6 +99,7 @@ _EXPORTS = [
     "frb_minmax_flat", "frb_normalize_flat", "frb_denormalize_flat", "frb_selftest_division",
     "frb_encode_workspace_size", "frb_encode_analyse", "frb_encode_emit", "frb_encode_index",
     "frb_decode_workspace_size", "frb_decode_batch", "frb_decode_tiles", "frb_decode_batch_indexed", "frb_decode_tiles_indexed",
+    "frb_decode_window", "frb_denormalize_window",
     "frb_probe_stream", "frb_debug_spin", "frb_parse_tile_headers", "frb_gather_seek_index",
     "frb_host_encode", "frb_host_decode",
     "frb_stream_encoder_new", "frb_stream_encoder_delete", "frb_stream_encoder_set_channels",
@@ -194,6 +201,8 @@ def lib():
     L.frb_encode_index.argtypes = [C.POINTER(EncodeParams), vp, sz, vp, vp, vp]
     L.frb_decode_batch_indexed.argtypes = [C.POINTER(DecodeParams), vp, vp, u64, vp, vp, vp, vp, sz, vp, vp]
     L.frb_decode_tiles_indexed.argtypes = [C.POINTER(DecodeParams), vp, vp, u64, vp, vp, vp, vp, C.c_double, vp, C.c_int, u32, u32, u32, vp, sz, vp, vp]
+    L.frb_decode_window.argtypes = [C.POINTER(DecodeParams), vp, vp, u64, vp, vp, vp, vp, C.c_double, Tile, vp, C.c_int, vp, sz, vp, vp]
+    L.frb_denormalize_window.argtypes = [vp, vp, u32, u32, vp, vp, C.c_double, Tile, vp, C.c_int, u32, vp]
     L.frb_debug_spin.argtypes = [u32, u32, u64, vp]
     L.frb_parse_tile_headers.argtypes = [vp, vp, vp, u32, vp]
     L.frb_gather_seek_index.argtypes = [vp, vp, vp, u32, u32, u32, vp, vp, vp]

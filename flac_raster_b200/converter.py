@@ -178,6 +178,92 @@ class RasterFLACConverter:
             raise ValueError("No metadata found in FLAC file or sidecar file")
         return decode_tile_blobs([blob], [hdr], [metadata])[0], metadata
 
+    def read_window(self, flac_path_or_url, col_off: int, row_off: int, width: int, height: int):
+        """The pixels of one window of a FLAC raster file (local path or URL) -> ((bands, height, width) array in the
+        original dtype, metadata).  Only the frames that cover the window are decoded: the metadata chain is read first,
+        then, when the file carries the "frbI" seek index, only the byte range of those frames (one read, or one HTTP
+        range request).  A file without the index (e.g. one the reference wrote) is read whole and its frames are found by
+        the sync scan.  The metadata is the file's, with width, height, transform and bounds of the window, and
+        `frames_decoded`.  Only the decoded frames are validated: damage in a frame outside the window goes unnoticed."""
+        import torch
+        from . import _native as nat
+        from .engine import TORCH_DTYPES, default_engine, window_frames
+        from .remote import RemoteFile, is_remote_url
+        from .tiffio import window_transform
+
+        src = str(flac_path_or_url)
+        if is_remote_url(src):
+            rf = RemoteFile(src)
+
+            def read(start: int, n: int) -> bytes:
+                return rf.read_range(start, start + n - 1) if n > 0 else b""
+        else:
+            path = Path(src)
+
+            def read(start: int, n: int) -> bytes:
+                with open(path, "rb") as f:
+                    f.seek(start)
+                    return f.read(n)          # n = -1: to the end
+        hdr = flacfmt.read_header(read)
+        metadata = parse_metadata_tags(hdr.tags)
+        if not metadata and not is_remote_url(src) and Path(src).with_suffix(".json").exists():
+            metadata = json.loads(Path(src).with_suffix(".json").read_text())
+        if not metadata:
+            raise ValueError("No metadata found in FLAC file or sidecar file")
+        si = hdr.streaminfo
+        bands, bps, blocksize = si.channels, si.bits_per_sample, si.max_blocksize
+        W, H = int(metadata["width"]), int(metadata["height"])
+        if metadata["count"] != bands:
+            raise ValueError("band count in tags does not match the FLAC channel count")
+        col_off, row_off, width, height = int(col_off), int(row_off), int(width), int(height)
+        if width < 1 or height < 1 or col_off < 0 or row_off < 0 or col_off + width > W or row_off + height > H:
+            raise ValueError(f"window (col_off={col_off}, row_off={row_off}, width={width}, height={height}) "
+                             f"is not inside the {W} x {H} raster")
+        window = (col_off, row_off, width, height)
+        tiles = np.zeros(1, dtype=nat.TILE_DTYPE)
+        tiles[0] = (0, 0, H, W)
+        n_frames = (W * H + blocksize - 1) // blocksize
+        blk = hdr.applications.get(flacfmt.SEEK_INDEX_ID)
+        index = flacfmt.unpack_seek_index(blk, bands, blocksize, n_frames) if blk else None
+        dtype = np.dtype(metadata["dtype"])
+        scale = float(metadata.get("scale_factor") or (32767 if bps == 16 else 8388607))     # as flac_to_array
+        if bps == 16:
+            scale = 32767.0
+        minmax = np.array([[metadata["data_min"], metadata["data_max"]]], dtype=np.float64)
+        rates = np.array([si.sample_rate], dtype=np.uint32)
+        eng = default_engine()
+        out = torch.empty((bands, height, width), dtype=TORCH_DTYPES[str(dtype)], device=eng.device)
+
+        def to_device(blob: bytes) -> "torch.Tensor":
+            host = np.zeros(len(blob) + 64, dtype=np.uint8)
+            host[:len(blob)] = np.frombuffer(blob, dtype=np.uint8)
+            return torch.from_numpy(host).to(eng.device)
+
+        status = None
+        if index is not None:
+            run = window_frames(tiles, window, blocksize, [index[0]])[0]
+            blob = read(hdr.first_frame_offset + int(run["byte_offset"]), int(run["byte_length"]))
+            if len(blob) == int(run["byte_length"]):
+                status = eng.decode_window(to_device(blob), np.zeros(1, np.int64), np.array([len(blob)]), tiles, rates, minmax,
+                                           scale, window, out, bps, blocksize, index=index, runs_only=True)
+        if status is None or status[0] or status[1] or status[2]:
+            # no index, or one that does not describe the frames: every frame is needed to find the window's by scanning
+            blob = read(hdr.first_frame_offset, -1) if not is_remote_url(src) else rf.read_all()[hdr.first_frame_offset:]
+            status = eng.decode_window(to_device(blob), np.zeros(1, np.int64), np.array([len(blob)]), tiles, rates, minmax,
+                                       scale, window, out, bps, blocksize)
+        _raise_for_status(status)
+        res = out.cpu().numpy()
+        meta = dict(metadata)
+        tr = metadata.get("transform")
+        t6 = window_transform(tuple(tr[:6]), col_off, row_off) if tr else None
+        left, top = (t6[2], t6[5]) if t6 else (float(col_off), -float(row_off))
+        meta.update({"width": width, "height": height, "transform": affine9(t6) if t6 else tr,
+                     "bounds": {"left": left, "bottom": top + height * (t6[4] if t6 else -1.0),
+                                "right": left + width * (t6[0] if t6 else 1.0), "top": top},
+                     "window": {"col_off": col_off, "row_off": row_off, "width": width, "height": height},
+                     "frames_decoded": int(status[3])})
+        return res, meta
+
     # kept for signature compatibility with the reference (converter.py:263, :329)
     def _embed_metadata_in_flac(self, flac_path: Path, metadata: Dict):
         blob = Path(flac_path).read_bytes()

@@ -19,10 +19,15 @@ namespace frb {
 
 constexpr unsigned long long kNoPos = 0xFFFFFFFFFFFFFFFFull;
 
+// n_samples / n_frames: what is decoded of the stream.  A window read decodes a run of frames [first_frame, first_frame +
+// n_frames) of a stream of total_samples samples (total_frames frames); every other call decodes whole streams
+// (first_frame 0, the totals equal to the counts).
 struct DecStreamDev {
     uint64_t byte_offset, byte_length, n_samples;
     int64_t audio_base;
-    uint32_t sample_rate, frame_base, n_frames, pad;
+    uint32_t sample_rate, frame_base, n_frames, first_frame;
+    uint64_t total_samples;
+    uint32_t total_frames, pad;
 };
 
 struct FrameHdr {
@@ -94,7 +99,7 @@ __global__ void k_fill_u64(unsigned long long *p, uint64_t n, unsigned long long
 __device__ __forceinline__ void sync_candidate(const uint8_t *__restrict__ bytes, const DecStreamDev &st, uint64_t pos, uint64_t start,
                                                uint64_t end, uint32_t channels, uint32_t bps, uint32_t blocksize,
                                                unsigned long long *__restrict__ frame_pos, unsigned long long *__restrict__ frame_pos2,
-                                               unsigned long long *__restrict__ probe) {
+                                               unsigned long long *__restrict__ probe, unsigned long long *__restrict__ end_cand) {
     if (pos < start || pos + 8 > end) return;
     FrameHdr h;
     if (!parse_frame_header(bytes + pos, end - pos, st.sample_rate, bps, &h)) return;
@@ -106,14 +111,34 @@ __device__ __forceinline__ void sync_candidate(const uint8_t *__restrict__ bytes
         atomicAdd(&probe[1], 1ull);
     }
     if (!frame_pos) return;
-    if (h.number >= st.n_frames) return;
-    const uint64_t expect = (h.number + 1 < st.n_frames) ? blocksize : (st.n_samples - h.number * blocksize);
+    // frame numbers are absolute: a run keeps [first_frame, first_frame + n_frames] (the last one marks where the run ends)
+    if (h.number < st.first_frame || h.number >= st.total_frames || h.number > (uint64_t)st.first_frame + st.n_frames) return;
+    const uint64_t expect = (h.number + 1 < st.total_frames) ? blocksize : (st.total_samples - h.number * blocksize);
     if (h.blocksize != expect) return;
     // the two smallest candidate positions per frame number: cand[f] and cand2[f] (k_sync_resolve picks between them).
     // Every position other than the final minimum is at some point the larger side of an atomicMin exchange, so the
     // minimum of those larger sides is the second smallest.
-    const unsigned long long old = atomicMin(&frame_pos[st.frame_base + h.number], (unsigned long long)pos);
-    if (frame_pos2 && old != kNoPos && old != pos) atomicMin(&frame_pos2[st.frame_base + h.number], old > pos ? old : (unsigned long long)pos);
+    const uint64_t k = h.number - st.first_frame;
+    unsigned long long *c1 = k < st.n_frames ? &frame_pos[st.frame_base + k] : end_cand;
+    unsigned long long *c2 = k < st.n_frames ? (frame_pos2 ? &frame_pos2[st.frame_base + k] : nullptr) : end_cand + 1;
+    if (!c1) return;
+    const unsigned long long old = atomicMin(c1, (unsigned long long)pos);
+    if (c2 && old != kNoPos && old != pos) atomicMin(c2, old > pos ? old : (unsigned long long)pos);
+}
+
+// Scan path of a window read: the frame behind a run's last frame gives the run's end (candidates picked as in
+// k_sync_resolve).  Written into the stream's byte_length, so that every later kernel sees a stream that ends there; a run
+// whose end was not found gets length 0 and its last frame is reported missing.
+__global__ void k_run_end(DecStreamDev *__restrict__ streams, uint32_t n_streams, const unsigned long long *__restrict__ cand,
+                          const unsigned long long *__restrict__ end_cand) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_streams) return;
+    DecStreamDev &st = streams[i];
+    if ((uint64_t)st.first_frame + st.n_frames >= st.total_frames) return;      // the run reaches the end of the stream
+    unsigned long long c = end_cand[2 * i];
+    const unsigned long long prev = cand[st.frame_base + st.n_frames - 1], c2 = end_cand[2 * i + 1];
+    if (c != kNoPos && prev != kNoPos && c <= prev && c2 != kNoPos) c = c2;
+    st.byte_length = (c == kNoPos || c < st.byte_offset) ? 0 : c - st.byte_offset;
 }
 
 // A byte sequence inside some frame's payload can look like a frame header (sync code, plausible fields, CRC-8: about
@@ -145,7 +170,8 @@ __global__ void __launch_bounds__(256)
 k_sync_scan(const uint8_t *__restrict__ bytes, const DecStreamDev *__restrict__ streams, uint32_t channels,
             uint32_t bps, uint32_t blocksize, unsigned long long *__restrict__ frame_pos,
             unsigned long long *__restrict__ frame_pos2 /* optional: second smallest candidate per frame */,
-            unsigned long long *__restrict__ probe /* optional: [0]=max key, [1]=count */, uint32_t parts) {
+            unsigned long long *__restrict__ probe /* optional: [0]=max key, [1]=count */, uint32_t parts,
+            unsigned long long *__restrict__ run_end = nullptr /* window reads: 2 candidates per stream for the frame behind the run */) {
     // flattened grid, `parts` CTAs per stream (gridDim.y stops at 65535 streams)
     const uint32_t si = blockIdx.x / parts, part = blockIdx.x - si * parts;
     const DecStreamDev st = streams[si];
@@ -168,7 +194,8 @@ k_sync_scan(const uint8_t *__restrict__ bytes, const DecStreamDev *__restrict__ 
 #pragma unroll
             for (int k = 0; k < 4; k++)
                 if (hit & (0xFFu << (8 * k)))
-                    sync_candidate(bytes, st, 16 * q + 4 * j + k, start, end, channels, bps, blocksize, frame_pos, frame_pos2, probe);
+                    sync_candidate(bytes, st, 16 * q + 4 * j + k, start, end, channels, bps, blocksize, frame_pos, frame_pos2, probe,
+                                   run_end ? run_end + 2 * si : nullptr);
         }
     }
 }
@@ -248,6 +275,7 @@ struct DecWorkspace {
     unsigned long long *frame_cand;     // scan path: smallest and second smallest candidate per frame, 2 x (total_frames + 1)
     uint8_t *chassign;
     uint32_t *sub_bitoff;      // only used when channels > 1
+    unsigned long long *run_end;        // scan path of a window read: 2 candidates per stream for the frame behind its run
 };
 static inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 static inline size_t dec_ws_layout(uint32_t n_streams, uint32_t channels, uint64_t total_frames, void *base, DecWorkspace *w) {
@@ -263,6 +291,8 @@ static inline size_t dec_ws_layout(uint32_t n_streams, uint32_t channels, uint64
     off += align256((size_t)total_frames + 1);
     if (w) w->sub_bitoff = (uint32_t *)(b + off);
     off += align256(4 * (size_t)(total_frames * channels + 1));
+    if (w) w->run_end = (unsigned long long *)(b + off);
+    off += align256(16 * (size_t)n_streams);
     return off;
 }
 
@@ -275,36 +305,63 @@ extern "C" int frb_decode_workspace_size(const frb_decode_params *p, uint64_t to
 }
 
 namespace frb {
-static int decode_batch_impl(const frb_decode_params *p, const frb_decode_stream *h_streams,
-                             const uint8_t *d_bytes, uint64_t total_frames, int32_t *d_audio,
-                             void *d_workspace, size_t workspace_bytes, uint32_t *d_status, void *stream, const SinkCfg &sink,
-                             const uint32_t *d_frame_bytes = nullptr, const uint32_t *d_index_bitoff = nullptr) {
+static int decode_streams_impl(const frb_decode_params *p, const std::vector<DecStreamDev> &hs,
+                               const uint8_t *d_bytes, uint64_t total_frames, int32_t *d_audio,
+                               void *d_workspace, size_t workspace_bytes, uint32_t *d_status, void *stream, const SinkCfg &sink,
+                               const uint32_t *d_frame_bytes, const uint32_t *d_index_bitoff);
+
+static int check_decode_args(const frb_decode_params *p, const void *h_streams, const uint8_t *d_bytes, uint64_t total_frames,
+                             const int32_t *d_audio, const void *d_workspace, const uint32_t *d_status, const SinkCfg &sink,
+                             const uint32_t *d_frame_bytes, const uint32_t *d_index_bitoff) {
     if ((d_frame_bytes == nullptr) != (d_index_bitoff == nullptr) && p && p->channels > 1) return FRB_ERR_INVALID_ARG;
     if (!p || !h_streams || !d_bytes || (!d_audio && sink.dtype < 0) || !d_workspace || !d_status) return FRB_ERR_INVALID_ARG;
     if (p->n_streams == 0 || p->channels < 1 || p->channels > FRB_MAX_CHANNELS || p->blocksize < 16 ||
         p->blocksize > 65535 || p->bps < 4 || p->bps > 32) return FRB_ERR_INVALID_ARG;
     if (total_frames == 0 || total_frames > 0x7FFFFFFFull) return FRB_ERR_INVALID_ARG;
+    return FRB_OK;
+}
+
+static int decode_batch_impl(const frb_decode_params *p, const frb_decode_stream *h_streams,
+                             const uint8_t *d_bytes, uint64_t total_frames, int32_t *d_audio,
+                             void *d_workspace, size_t workspace_bytes, uint32_t *d_status, void *stream, const SinkCfg &sink,
+                             const uint32_t *d_frame_bytes = nullptr, const uint32_t *d_index_bitoff = nullptr) {
+    FRB_TRY(check_decode_args(p, h_streams, d_bytes, total_frames, d_audio, d_workspace, d_status, sink, d_frame_bytes, d_index_bitoff));
+    // stream table (host -> device). Pageable source: staged by the runtime before return.
+    std::vector<DecStreamDev> hs(p->n_streams);
+    uint64_t frames = 0;
+    for (uint32_t i = 0; i < p->n_streams; i++) {
+        const frb_decode_stream &a = h_streams[i];
+        DecStreamDev d;
+        d.byte_offset = a.byte_offset; d.byte_length = a.byte_length; d.n_samples = a.n_samples;
+        d.audio_base = a.audio_base; d.sample_rate = a.sample_rate; d.frame_base = a.frame_base;
+        d.n_frames = (uint32_t)((a.n_samples + p->blocksize - 1) / p->blocksize);
+        d.first_frame = 0; d.total_samples = d.n_samples; d.total_frames = d.n_frames; d.pad = 0;
+        if (a.frame_base != frames) return FRB_ERR_INVALID_ARG;
+        frames += d.n_frames;
+        hs[i] = d;
+    }
+    if (frames != total_frames) return FRB_ERR_INVALID_ARG;
+    return decode_streams_impl(p, hs, d_bytes, total_frames, d_audio, d_workspace, workspace_bytes, d_status, stream, sink,
+                               d_frame_bytes, d_index_bitoff);
+}
+
+// the work of every decode call, on a stream table that holds whole streams or frame runs (DecStreamDev)
+static int decode_streams_impl(const frb_decode_params *p, const std::vector<DecStreamDev> &hs,
+                               const uint8_t *d_bytes, uint64_t total_frames, int32_t *d_audio,
+                               void *d_workspace, size_t workspace_bytes, uint32_t *d_status, void *stream, const SinkCfg &sink,
+                               const uint32_t *d_frame_bytes, const uint32_t *d_index_bitoff) {
     int rc = ensure_tables_impl();
     if (rc) return rc;
     DecWorkspace w;
     if (dec_ws_layout(p->n_streams, p->channels, total_frames, d_workspace, &w) > workspace_bytes) return FRB_ERR_OVERFLOW;
     if (reinterpret_cast<uintptr_t>(d_bytes) & 15u) return FRB_ERR_INVALID_ARG;   // vector loads need a 16-byte aligned base
     cudaStream_t s = (cudaStream_t)stream;
-    // stream table (host -> device). Pageable source: staged by the runtime before return.
-    std::vector<DecStreamDev> hs(p->n_streams);
-    uint64_t max_len = 0, frames = 0;
-    for (uint32_t i = 0; i < p->n_streams; i++) {
-        const frb_decode_stream &a = h_streams[i];
-        DecStreamDev d;
-        d.byte_offset = a.byte_offset; d.byte_length = a.byte_length; d.n_samples = a.n_samples;
-        d.audio_base = a.audio_base; d.sample_rate = a.sample_rate; d.frame_base = a.frame_base;
-        d.n_frames = (uint32_t)((a.n_samples + p->blocksize - 1) / p->blocksize); d.pad = 0;
-        if (a.frame_base != frames) return FRB_ERR_INVALID_ARG;
-        frames += d.n_frames;
-        if (a.byte_length > max_len) max_len = a.byte_length;
-        hs[i] = d;
+    uint64_t max_len = 0;
+    bool open_runs = false;                  // a run that ends before its stream does (scan path: k_run_end finds its end)
+    for (const DecStreamDev &d : hs) {
+        if (d.byte_length > max_len) max_len = d.byte_length;
+        if ((uint64_t)d.first_frame + d.n_frames < d.total_frames) open_runs = true;
     }
-    if (frames != total_frames) return FRB_ERR_INVALID_ARG;
     FRB_TRY(small_upload(w.streams, hs.data(), sizeof(DecStreamDev) * hs.size(), s));   // staged in pinned memory before returning
     FRB_TRY(small_fill(d_status, 0u, 8 * sizeof(uint32_t), s));
     FRB_TRY(small_fill(w.chassign, 0u, ((size_t)total_frames + 1 + 3) & ~(size_t)3, s));
@@ -317,6 +374,10 @@ static int decode_batch_impl(const frb_decode_params *p, const frb_decode_stream
     } else {
         k_fill_u64<<<grid_for(2 * (total_frames + 1), 256 * 4, kNumSMs * 4), 256, 0, s>>>(w.frame_cand, 2 * (total_frames + 1), kNoPos);
         FRB_LAUNCH_CHECK("k_fill_u64");
+        if (open_runs) {
+            k_fill_u64<<<1, 256, 0, s>>>(w.run_end, 2 * (uint64_t)p->n_streams, kNoPos);
+            FRB_LAUNCH_CHECK("k_fill_u64");
+        }
         uint64_t chunks = max_len / 16 + 2;
         uint32_t gx = (uint32_t)((chunks + 256 * 4 - 1) / (256 * 4));
         uint32_t cap = (kNumSMs * 16 + p->n_streams - 1) / p->n_streams;
@@ -324,12 +385,16 @@ static int decode_batch_impl(const frb_decode_params *p, const frb_decode_stream
         if (gx < 1) gx = 1;
         prof_begin(3, s);
         k_sync_scan<<<gx * p->n_streams, 256, 0, s>>>(d_bytes, w.streams, p->channels, p->bps, p->blocksize, w.frame_cand,
-                                                      w.frame_cand + total_frames + 1, nullptr, gx);
+                                                      w.frame_cand + total_frames + 1, nullptr, gx, open_runs ? w.run_end : nullptr);
         prof_end(3, s);
         FRB_LAUNCH_CHECK("k_sync_scan");
         k_sync_resolve<<<(uint32_t)((total_frames + 255) / 256), 256, 0, s>>>(w.streams, p->n_streams, (uint32_t)total_frames, w.frame_cand,
                                                                             w.frame_cand + total_frames + 1, w.frame_pos);
         FRB_LAUNCH_CHECK("k_sync_resolve");
+        if (open_runs) {
+            k_run_end<<<(p->n_streams + 255) / 256, 256, 0, s>>>(w.streams, p->n_streams, w.frame_cand, w.run_end);
+            FRB_LAUNCH_CHECK("k_run_end");
+        }
     }
     // CRC-16 only needs the frame positions: it runs on a side stream and joins the caller's stream at the end.  It is launched
     // AFTER the decode kernel: CTAs of the earlier launch are placed first, so the CRC's CTAs fill the SMs only as the decode grid
@@ -390,12 +455,13 @@ static int decode_batch_impl(const frb_decode_params *p, const frb_decode_stream
         if (two_env < 0) { const char *e = getenv("FRB_DECODE_TWO_LAUNCH"); two_env = e ? atoi(e) : 0; }
         const bool two_launch = n_skim_ctas > 0 && ((p->verify_crc16 & 2u) || two_env);
         prof_begin(1, s);
-#define FRB_DECODE(BIG, RAS, GRID, NSKIM) k_decode_subframes<BIG, RAS><<<GRID, kDecThreads, 0, s>>>(d_bytes, w.streams, p->n_streams, p->channels, p->bps, \
+#define FRB_DECODE(BIG, SINK, GRID, NSKIM) k_decode_subframes<BIG, SINK><<<GRID, kDecThreads, 0, s>>>(d_bytes, w.streams, p->n_streams, p->channels, p->bps, \
             p->blocksize, (uint32_t)total_frames, w.frame_pos, sub_bitoff, d_audio, w.chassign, d_status, NSKIM, skim_lanes, sink, \
             indexed ? 1u : 0u)
 #define FRB_DECODE_ANY(GRID, NSKIM) do { \
-        if (sink.dtype < 0) { if (big) FRB_DECODE(true, false, GRID, NSKIM); else FRB_DECODE(false, false, GRID, NSKIM); } \
-        else { if (big) FRB_DECODE(true, true, GRID, NSKIM); else FRB_DECODE(false, true, GRID, NSKIM); } } while (0)
+        if (sink.dtype < 0) { if (big) FRB_DECODE(true, kSinkAudio, GRID, NSKIM); else FRB_DECODE(false, kSinkAudio, GRID, NSKIM); } \
+        else if (!sink.window) { if (big) FRB_DECODE(true, kSinkTile, GRID, NSKIM); else FRB_DECODE(false, kSinkTile, GRID, NSKIM); } \
+        else { if (big) FRB_DECODE(true, kSinkWindow, GRID, NSKIM); else FRB_DECODE(false, kSinkWindow, GRID, NSKIM); } } while (0)
         if (two_launch) {
             FRB_DECODE_ANY(n_skim_ctas, n_skim_ctas);          // a grid of skim CTAs only
             FRB_LAUNCH_CHECK("k_decode_subframes(skim)");
@@ -442,6 +508,7 @@ static int frb_decode_tiles_impl(const frb_decode_params *p, const frb_decode_st
     if (p->channels == 2) return FRB_ERR_UNSUPPORTED;
     static const uint32_t esz[8] = {1, 1, 2, 2, 4, 4, 4, 8};
     SinkCfg sink;
+    memset(&sink, 0, sizeof sink);
     sink.dtype = dtype; sink.esize = esz[dtype]; sink.H = H; sink.W = W; sink.tiles = d_tiles; sink.minmax = d_minmax;
     sink.raster = (uint8_t *)d_raster; sink.scale = scale; sink.rcp = 1.0 / scale;
     sink.fast = (scale == 32767.0 || scale == 8388607.0 || scale == 2147483647.0) ? 1 : 0;
@@ -480,6 +547,63 @@ extern "C" int frb_decode_batch_indexed(const frb_decode_params *p, const frb_de
     sink.dtype = -1;
     return frb::decode_batch_impl(p, h_streams, d_bytes, total_frames, d_audio, d_workspace, workspace_bytes, d_status, stream, sink,
                                   d_frame_bytes, d_sub_bitoff);
+}
+
+extern "C" int frb_decode_window(const frb_decode_params *p, const frb_window_stream *h_streams,
+                                 const uint8_t *d_bytes, uint64_t total_frames,
+                                 const uint32_t *d_frame_bytes, const uint32_t *d_sub_bitoff,
+                                 const frb_tile *d_tiles, const double *d_minmax, double scale, frb_tile window,
+                                 void *d_out, int dtype, void *d_workspace, size_t workspace_bytes, uint32_t *d_status, void *stream) {
+    using namespace frb;
+    if (!p || !d_out || dtype < -1 || dtype > FRB_F64) return FRB_ERR_INVALID_ARG;
+    if (dtype >= 0 && (!d_tiles || !d_minmax || !(scale > 0.0) || window.h == 0 || window.w == 0)) return FRB_ERR_INVALID_ARG;
+    if (dtype >= 0 && p->channels == 2) return FRB_ERR_UNSUPPORTED;       // mid/side frames: dtype -1 + frb_denormalize_window
+    SinkCfg sink;
+    memset(&sink, 0, sizeof sink);
+    sink.dtype = -1;
+    if (dtype >= 0) {
+        static const uint32_t esz[8] = {1, 1, 2, 2, 4, 4, 4, 8};
+        sink.dtype = dtype; sink.esize = esz[dtype]; sink.H = window.h; sink.W = window.w; sink.tiles = d_tiles; sink.minmax = d_minmax;
+        sink.raster = (uint8_t *)d_out; sink.scale = scale; sink.rcp = 1.0 / scale;
+        sink.fast = (scale == 32767.0 || scale == 8388607.0 || scale == 2147483647.0) ? 1 : 0;
+        sink.intpath = (dtype <= FRB_I16 && scale == 32767.0) ? 1 : 0;
+        sink.window = 1; sink.win_row = window.row_off; sink.win_col = window.col_off;
+    }
+    int32_t *d_audio = dtype < 0 ? (int32_t *)d_out : nullptr;
+    FRB_TRY(check_decode_args(p, h_streams, d_bytes, total_frames, d_audio, d_workspace, d_status, sink, d_frame_bytes, d_sub_bitoff));
+    std::vector<DecStreamDev> hs(p->n_streams);
+    uint64_t frames = 0;
+    for (uint32_t i = 0; i < p->n_streams; i++) {
+        const frb_window_stream &a = h_streams[i];
+        DecStreamDev d;
+        const uint64_t all = (a.total_samples + p->blocksize - 1) / p->blocksize;
+        if (a.n_frames == 0 || all > 0xFFFFFFFFull || (uint64_t)a.first_frame + a.n_frames > all || a.frame_base != frames)
+            return FRB_ERR_INVALID_ARG;
+        const uint64_t s0 = (uint64_t)a.first_frame * p->blocksize, s1 = (uint64_t)(a.first_frame + a.n_frames) * p->blocksize;
+        d.byte_offset = a.byte_offset; d.byte_length = a.byte_length;
+        d.n_samples = (s1 < a.total_samples ? s1 : a.total_samples) - s0;
+        d.audio_base = a.audio_base; d.sample_rate = a.sample_rate; d.frame_base = a.frame_base; d.n_frames = a.n_frames;
+        d.first_frame = a.first_frame; d.total_samples = a.total_samples; d.total_frames = (uint32_t)all; d.pad = 0;
+        frames += a.n_frames;
+        hs[i] = d;
+    }
+    if (frames != total_frames) return FRB_ERR_INVALID_ARG;
+    return decode_streams_impl(p, hs, d_bytes, total_frames, d_audio, d_workspace, workspace_bytes, d_status, stream, sink,
+                               d_frame_bytes, d_sub_bitoff);
+}
+
+extern "C" int frb_denormalize_window(const int32_t *d_audio, const frb_window_stream *d_streams, uint32_t n_tiles, uint32_t blocksize,
+                                      const frb_tile *d_tiles, const double *d_minmax, double scale, frb_tile window,
+                                      void *d_out, int dtype, uint32_t bands, void *stream) {
+    using namespace frb;
+    if (!d_audio || !d_streams || !d_tiles || !d_minmax || !d_out || dtype < 0 || dtype > FRB_F64 || !bands || !n_tiles ||
+        !blocksize || !(scale > 0.0) || window.h == 0 || window.w == 0) return FRB_ERR_INVALID_ARG;
+    cudaStream_t s = (cudaStream_t)stream;
+    const uint32_t parts = tile_grid_parts(n_tiles, bands * window.h), grid = parts * n_tiles;
+    FRB_DISPATCH_DTYPE(dtype, (k_denormalize_window<T><<<grid, kMapThreads, 0, s>>>(d_audio, d_streams, blocksize, d_tiles, d_minmax, scale,
+                                                                                   window, (T *)d_out, bands, parts)));
+    FRB_LAUNCH_CHECK("k_denormalize_window");
+    return FRB_OK;
 }
 
 #ifdef FRB_DEC_TIMING

@@ -524,13 +524,20 @@ struct SinkCfg {
     double scale, rcp;
     int fast;                // scale is one of the three reference constants (exact reciprocal division)
     int intpath;             // 8/16-bit integer raster + scale 32767: exact integer evaluation of the fp64 formula (sink_px)
+    int window;              // window sink (frb_decode_window): raster is the (bands, H, W) window at image (win_row, win_col)
+    uint32_t win_row, win_col;
 };
+// output of k_decode_subframes: planar int32 audio, the tiles' windows of a raster, or the part of them inside a window
+constexpr int kSinkAudio = 0, kSinkTile = 1, kSinkWindow = 2;
 struct RasterPos {           // per thread
     uint8_t *rowp;           // first pixel of the current row of this tile/band window
     uint32_t x, w, pitch;    // position inside the row, row length (pixels), raster row pitch in bytes
     double mn, range;        // fp64 path
     int32_t imn;             // integer path: data_min - 1, data_max - data_min (integers for integer rasters, range < 2^16)
     uint32_t irange, kround; // kround = 32767*range + 32767 + 65534 (see sink_px)
+    // window sink: rowp/x address the current tile row as if the whole row were stored (x = column in the tile); only
+    // rows [y0, y1) and columns [x0, x1) of the tile lie inside the window and are stored
+    uint32_t y, y0, y1, x0, x1;
 };
 
 typedef BitReader DecReader;
@@ -566,13 +573,16 @@ __device__ __forceinline__ uint32_t sink_px(const RasterPos &R, int32_t a, bool 
 __device__ __noinline__ uint32_t sink_px_tie(double scale, double rcp, int32_t imn_minus_1, uint32_t irange, int32_t a) {
     return (uint32_t)(int32_t)__double2ll_rn(denormalize_one_fast((double)a, scale, rcp, (double)(imn_minus_1 + 1), (double)irange));
 }
-__device__ __forceinline__ void sink_put1(const SinkCfg &G, RasterPos &R, int32_t a) {
+__device__ __forceinline__ void sink_store1(const SinkCfg &G, const RasterPos &R, int32_t a) {
     if (G.intpath) {
         bool tie = false;
         uint32_t v = sink_px(R, a, tie);
         if (tie) v = sink_px_tie(G.scale, G.rcp, R.imn, R.irange, a);
         if (G.esize == 2) reinterpret_cast<uint16_t *>(R.rowp)[R.x] = (uint16_t)v; else R.rowp[R.x] = (uint8_t)v;
     } else store_denorm(R.rowp, G.dtype, R.x, sink_map(G, R, a));
+}
+__device__ __forceinline__ void sink_put1(const SinkCfg &G, RasterPos &R, int32_t a) {
+    sink_store1(G, R, a);
     if (++R.x == R.w) { R.x = 0; R.rowp += R.pitch; }
 }
 // rare slow path of sink_put_batch (a sample on an exact rounding tie, or a batch that straddles a row end): kept out of
@@ -707,6 +717,32 @@ __device__ __forceinline__ void sink_put_batch(const SinkCfg &G, RasterPos &R, c
     }
 }
 
+// ---- window sink: the tile sink clipped to a window -------------------------------------------------
+__device__ __forceinline__ bool win_row_visible(const RasterPos &R) { return R.y - R.y0 < R.y1 - R.y0; }
+__device__ __forceinline__ void win_put1(const SinkCfg &G, RasterPos &R, int32_t a) {
+    if (win_row_visible(R) && R.x - R.x0 < R.x1 - R.x0) sink_store1(G, R, a);
+    if (++R.x == R.w) { R.x = 0; R.y++; R.rowp += R.pitch; }
+}
+// A batch inside the row's visible span takes the tile sink's vector stores; a batch inside a row outside the window
+// only moves the position; the rest (batches across a row end or a window edge) goes sample by sample.
+__device__ __forceinline__ void win_put_batch(const SinkCfg &G, RasterPos &R, const int32_t (&a)[kDecBatch]) {
+    const bool vis = win_row_visible(R);
+    if (vis && R.x >= R.x0 && R.x + kDecBatch <= R.x1) {
+        sink_put_batch(G, R, a);                 // inside the row: never straddles, wraps to x = 0 at the row end
+        if (R.x == 0) R.y++;
+    } else if (!vis && R.x + kDecBatch <= R.w) {
+        R.x += kDecBatch;
+        if (R.x == R.w) { R.x = 0; R.y++; R.rowp += R.pitch; }
+    } else {
+#pragma unroll 1
+        for (int j = 0; j < kDecBatch; j++) win_put1(G, R, a[j]);
+    }
+}
+template <int SINK>
+__device__ __forceinline__ void sink_one(const SinkCfg &G, RasterPos &R, int32_t a) {
+    if constexpr (SINK == kSinkWindow) win_put1(G, R, a); else sink_put1(G, R, a);
+}
+
 // FIXED / LPC subframe, part 1 (per lane, divergent): warm-up samples, predictor, residual coding header and the
 // first partition's parameter.  Run BEFORE the warp picks its sample loop, so that the loop can use libFLAC's
 // 32-bit rule with the subframe's ACTUAL coefficient precision (16-bit audio coded by libFLAC has precision <= 12
@@ -719,7 +755,7 @@ struct PredState {
     uint32_t k, plen, esc, psize, part_left, raw_bits, i;
     bool escape, wide;
 };
-template <int PMAX, bool RASTER>
+template <int PMAX, int SINK>
 __device__ __forceinline__ void decode_prologue(SubCtx &S, bool active, PredState<PMAX> &P, const SinkCfg &G) {
     DecReader &br = S.br;
     const uint32_t n = S.n, order = S.order, wasted = S.wasted;
@@ -734,7 +770,7 @@ __device__ __forceinline__ void decode_prologue(SubCtx &S, bool active, PredStat
         for (int q = 0; q < PMAX - 1; q++) P.hist[q] = P.hist[q + 1];
         P.hist[PMAX - 1] = v;
         const int32_t sv = shl_checked(v, wasted, S.err);
-        if (!RASTER) S.dst[w] = sv; else sink_put1(G, S.rp, sv);
+        if (SINK == kSinkAudio) S.dst[w] = sv; else sink_one<SINK>(G, S.rp, sv);
     }
     br.top_up();
     if (S.type == 3) {
@@ -778,7 +814,7 @@ __device__ __forceinline__ void decode_prologue(SubCtx &S, bool active, PredStat
 // data-dependent branches (predicated word merges, see BitReader) followed by the predictor recursion from the
 // register history, or a single sample through the generic path (escape-coded partitions, partition tails, codes
 // longer than 32 bits).
-template <int MAXORD, bool WIDE, int PMAX, bool RASTER>
+template <int MAXORD, bool WIDE, int PMAX, int SINK>
 __device__ __forceinline__ void decode_predictive(SubCtx &S, const PredState<PMAX> &P, const SinkCfg &G) {
     DecReader &br = S.br;
     const uint32_t n = S.n, wasted = S.wasted;
@@ -830,11 +866,11 @@ __device__ __forceinline__ void decode_predictive(SubCtx &S, const PredState<PMA
         }
     };
     auto output_batch = [&]() {
-        if (RASTER) {
+        if (SINK != kSinkAudio) {
             int32_t o[kDecBatch];
 #pragma unroll
             for (int j = 0; j < kDecBatch; j++) o[j] = (int32_t)((uint32_t)H[MAXORD + j] << wasted);
-            sink_put_batch(G, S.rp, o);
+            if constexpr (SINK == kSinkWindow) win_put_batch(G, S.rp, o); else sink_put_batch(G, S.rp, o);
         } else if (S.aligned16) {
 #pragma unroll
             for (int q = 0; q < kDecBatch / 4; q++)
@@ -860,7 +896,7 @@ __device__ __forceinline__ void decode_predictive(SubCtx &S, const PredState<PMA
 #pragma unroll
         for (int q = 0; q < MAXORD - 1; q++) H[q] = H[q + 1];
         H[MAXORD - 1] = v;
-        if (!RASTER) dst[i] = (int32_t)((uint32_t)v << wasted); else sink_put1(G, S.rp, (int32_t)((uint32_t)v << wasted));
+        if (SINK == kSinkAudio) dst[i] = (int32_t)((uint32_t)v << wasted); else sink_one<SINK>(G, S.rp, (int32_t)((uint32_t)v << wasted));
         part_left--; i++;
         if (br.overrun()) { S.err = true; i = n; }
     };
@@ -909,7 +945,7 @@ constexpr uint32_t kSpinLimit = 1u << 22;
 #ifdef FRB_DEC_TIMING
 __device__ unsigned long long g_dec_dbg[16];
 #endif
-template <bool BIGORDER, bool RASTER>
+template <bool BIGORDER, int SINK>
 __global__ void __launch_bounds__(kDecThreads, BIGORDER ? 1 : FRB_DEC_MINB)
 k_decode_subframes(const uint8_t *__restrict__ bytes, const DecStreamDev *__restrict__ streams, uint32_t n_streams,
                    uint32_t channels, uint32_t bps, uint32_t blocksize, uint32_t total_frames,
@@ -941,7 +977,7 @@ k_decode_subframes(const uint8_t *__restrict__ bytes, const DecStreamDev *__rest
     const uint32_t c = alive ? s / total_frames : 0, f = alive ? s - c * total_frames : 0;
     SubCtx S;
     S.err = false; S.type = 0; S.order = 0; S.n = 0; S.wasted = 0; S.sbps = bps; S.dst = audio; S.aligned16 = false;
-    S.rp.rowp = sink.raster; S.rp.x = 0; S.rp.w = 1; S.rp.pitch = 0; S.rp.mn = 0.0; S.rp.range = 0.0; S.rp.imn = 0; S.rp.irange = 0; S.rp.kround = 0;
+    S.rp.rowp = sink.raster; S.rp.x = 0; S.rp.w = 1; S.rp.y = S.rp.y0 = S.rp.y1 = S.rp.x0 = S.rp.x1 = 0; S.rp.pitch = 0; S.rp.mn = 0.0; S.rp.range = 0.0; S.rp.imn = 0; S.rp.irange = 0; S.rp.kround = 0;
     S.br.gq = (const uint4 *)bytes; S.br.sbase = (uint32_t)__cvta_generic_to_shared(s_ring + threadIdx.x * kSkimRing);
     S.br.swz = (lane & 15u) << 4; S.br.sx = S.br.sbase ^ S.br.swz; S.br.cissue = 0; S.br.qlast = 0;
     S.br.woff = 12; S.br.A = S.br.B = S.br.Craw = 0; S.br.bp = 0;
@@ -983,7 +1019,27 @@ k_decode_subframes(const uint8_t *__restrict__ bytes, const DecStreamDev *__rest
                 const int64_t idx = st.audio_base + (int64_t)c * (int64_t)st.n_samples + (int64_t)L.k * blocksize;
                 S.dst = audio + idx;
                 S.aligned16 = ((reinterpret_cast<uintptr_t>(S.dst) & 15u) == 0);
-                if (RASTER) {
+                if (SINK == kSinkWindow) {
+                    const frb_tile t = sink.tiles[L.stream];
+                    if ((uint64_t)t.h * t.w != st.total_samples || t.w == 0) {
+                        if (c == 0 && L.k == 0) atomicAdd(&status[6], 1u);
+                        alive = false;
+                    }
+                    const uint64_t i0 = (uint64_t)(st.first_frame + L.k) * blocksize;
+                    const uint32_t y = t.w ? (uint32_t)(i0 / t.w) : 0u;
+                    // the window in tile coordinates, clipped to the tile
+                    const int64_t wy = (int64_t)sink.win_row - t.row_off, wx = (int64_t)sink.win_col - t.col_off;
+                    auto clip = [](int64_t v, uint32_t hi) -> uint32_t { return (uint32_t)(v < 0 ? 0 : v > (int64_t)hi ? (int64_t)hi : v); };
+                    S.rp.y = y; S.rp.y0 = clip(wy, t.h); S.rp.y1 = clip(wy + sink.H, t.h);
+                    S.rp.x0 = clip(wx, t.w); S.rp.x1 = clip(wx + sink.W, t.w);
+                    S.rp.x = (uint32_t)(i0 - (uint64_t)y * t.w); S.rp.w = t.w; S.rp.pitch = sink.W * sink.esize;
+                    // row y of the tile, column 0 (outside the window unless its rows and columns are: only ever offset)
+                    S.rp.rowp = sink.raster + (((int64_t)c * sink.H + (int64_t)y - wy) * (int64_t)sink.W - wx) * (int64_t)sink.esize;
+                    const double mn = sink.minmax[2 * L.stream];
+                    const double range = __dsub_rn(sink.minmax[2 * L.stream + 1], mn);
+                    if (sink.intpath) { S.rp.imn = (int32_t)mn - 1; S.rp.irange = (uint32_t)range; S.rp.kround = 32767u * S.rp.irange + 32767u + 65534u; }
+                    else { S.rp.mn = mn; S.rp.range = range; }
+                } else if (SINK == kSinkTile) {
                     const frb_tile t = sink.tiles[L.stream];
                     // the stream must be exactly this tile's pixels and the window must lie inside the raster (status[6])
                     if ((uint64_t)t.h * t.w != st.n_samples || t.w == 0 || (uint64_t)t.row_off + t.h > sink.H || (uint64_t)t.col_off + t.w > sink.W) {
@@ -1018,13 +1074,13 @@ k_decode_subframes(const uint8_t *__restrict__ bytes, const DecStreamDev *__rest
     if (run) {
         if (S.type == 0) {
             const int32_t v = shl_checked(S.br.get_signed(S.sbps, &S.err), S.wasted, S.err);
-            if (!RASTER) { for (uint32_t i = 0; i < S.n; i++) S.dst[i] = v; }
-            else { for (uint32_t i = 0; i < S.n; i++) sink_put1(sink, S.rp, v); }
+            if (SINK == kSinkAudio) { for (uint32_t i = 0; i < S.n; i++) S.dst[i] = v; }
+            else { for (uint32_t i = 0; i < S.n; i++) sink_one<SINK>(sink, S.rp, v); }
         } else if (S.type == 1) {
             for (uint32_t i = 0; i < S.n; i++) {
                 if ((i & 3u) == 0) S.br.top_up();
                 const int32_t v = shl_checked(S.br.get_signed(S.sbps, &S.err), S.wasted, S.err);
-                if (!RASTER) S.dst[i] = v; else sink_put1(sink, S.rp, v);
+                if (SINK == kSinkAudio) S.dst[i] = v; else sink_one<SINK>(sink, S.rp, v);
             }
         } else if (!BIGORDER && S.order > 12) {
             S.err = true;
@@ -1035,15 +1091,15 @@ k_decode_subframes(const uint8_t *__restrict__ bytes, const DecStreamDev *__rest
         constexpr int PMAX = BIGORDER ? 32 : 12;
         const bool act = run && S.type >= 2 && (BIGORDER || S.order <= 12);
         PredState<PMAX> P;
-        decode_prologue<PMAX, RASTER>(S, act, P, sink);
+        decode_prologue<PMAX, SINK>(S, act, P, sink);
         // warp-uniform sample loop (it is warp-synchronous): taps padded to the largest order in the warp, 64-bit MACs
         // only if a lane needs them
         const uint32_t cls = __reduce_max_sync(0xFFFFFFFFu, act ? S.order : 0u);
         const bool wide = __any_sync(0xFFFFFFFFu, act && P.wide);
-        if (BIGORDER) decode_predictive<32, true, PMAX, RASTER>(S, P, sink);
-        else if (cls <= 4) { if (wide) decode_predictive<4, true, PMAX, RASTER>(S, P, sink); else decode_predictive<4, false, PMAX, RASTER>(S, P, sink); }
-        else if (cls <= 8) { if (wide) decode_predictive<8, true, PMAX, RASTER>(S, P, sink); else decode_predictive<8, false, PMAX, RASTER>(S, P, sink); }
-        else { if (wide) decode_predictive<12, true, PMAX, RASTER>(S, P, sink); else decode_predictive<12, false, PMAX, RASTER>(S, P, sink); }
+        if (BIGORDER) decode_predictive<32, true, PMAX, SINK>(S, P, sink);
+        else if (cls <= 4) { if (wide) decode_predictive<4, true, PMAX, SINK>(S, P, sink); else decode_predictive<4, false, PMAX, SINK>(S, P, sink); }
+        else if (cls <= 8) { if (wide) decode_predictive<8, true, PMAX, SINK>(S, P, sink); else decode_predictive<8, false, PMAX, SINK>(S, P, sink); }
+        else { if (wide) decode_predictive<12, true, PMAX, SINK>(S, P, sink); else decode_predictive<12, false, PMAX, SINK>(S, P, sink); }
     }
 #ifdef FRB_DEC_TIMING
     {

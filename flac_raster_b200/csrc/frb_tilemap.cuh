@@ -401,6 +401,52 @@ k_denormalize_tiles(const int32_t *__restrict__ audio, const int64_t *__restrict
     }
 }
 
+// The window read's gather (frb_denormalize_window): audio of frame runs (frb_decode_window, dtype -1) -> the part of every
+// tile that lies inside the window.  `parts` CTAs per tile, a warp per (band, visible row), a thread per group of G
+// pixels; the same per-sample mapping as k_denormalize_tiles.
+template <typename T>
+__global__ void __launch_bounds__(kMapThreads)
+k_denormalize_window(const int32_t *__restrict__ audio, const frb_window_stream *__restrict__ streams, uint32_t blocksize,
+                     const frb_tile *__restrict__ tiles, const double *__restrict__ minmax, double scale, frb_tile win,
+                     T *__restrict__ out_all, uint32_t bands, uint32_t parts) {
+    constexpr int G = MapGroup<T>::G;
+    const uint32_t tile_i = blockIdx.x / parts, part = blockIdx.x - tile_i * parts;
+    const frb_tile t = tiles[tile_i];
+    const frb_window_stream st = streams[tile_i];
+    // visible rows / columns in tile coordinates
+    const int64_t wy = (int64_t)win.row_off - t.row_off, wx = (int64_t)win.col_off - t.col_off;
+    auto clip = [](int64_t v, uint32_t hi) -> uint32_t { return (uint32_t)(v < 0 ? 0 : v > (int64_t)hi ? (int64_t)hi : v); };
+    const uint32_t y0 = clip(wy, t.h), y1 = clip(wy + win.h, t.h), x0 = clip(wx, t.w), x1 = clip(wx + win.w, t.w);
+    if (y0 >= y1 || x0 >= x1) return;
+    const uint64_t s0 = (uint64_t)st.first_frame * blocksize, s1 = (uint64_t)(st.first_frame + st.n_frames) * blocksize;
+    const uint64_t run_n = (s1 < st.total_samples ? s1 : st.total_samples) - s0;
+    const double mn = minmax[2 * tile_i], mx = minmax[2 * tile_i + 1];
+    const double range = __dsub_rn(mx, mn);
+    const bool fast = scale == 32767.0 || scale == 8388607.0 || scale == 2147483647.0;
+    const double rcp = __drcp_rn(scale);
+    auto map = [&](int32_t a) -> T {
+        return denorm_cast<T>(fast ? denormalize_one_fast((double)a, scale, rcp, mn, range) : denormalize_one((double)a, scale, mn, range));
+    };
+    const uint32_t vh = y1 - y0, vw = x1 - x0, rows = bands * vh;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (uint32_t ry = part * kMapWarps + warp; ry < rows; ry += parts * kMapWarps) {
+        const uint32_t c = ry / vh, y = y0 + (ry - c * vh);
+        T *out = out_all + ((size_t)c * win.h + (size_t)((int64_t)y - wy)) * win.w + (size_t)((int64_t)x0 - wx);
+        const int32_t *in = audio + st.audio_base + (int64_t)((size_t)c * run_n + ((uint64_t)y * t.w + x0 - s0));
+        const RowSplit<T> rs(out, vw);
+        if ((uint32_t)lane < rs.head) out[lane] = map(in[lane]);
+        if (rs.tail0 + lane < vw) out[rs.tail0 + lane] = map(in[rs.tail0 + lane]);
+        T *obody = out + rs.head;
+        const int32_t *ibody = in + rs.head;
+        for (uint32_t g = lane; g < rs.ngroups; g += 32) {
+            T e[G];
+#pragma unroll
+            for (int j = 0; j < G; j++) e[j] = map(__ldcs(ibody + (size_t)g * G + j));
+            store_group(obody + (size_t)g * G, e);
+        }
+    }
+}
+
 static inline uint32_t tile_grid_parts(uint32_t n_tiles, uint32_t max_rows) {
     // ~16 CTAs per SM in total, but never more CTAs per tile than it has (band,row) groups of kMapWarps
     uint32_t per_tile = (kNumSMs * 16 + n_tiles - 1) / n_tiles;

@@ -47,6 +47,52 @@ def _check_tile_sizes(npx: np.ndarray) -> None:
         raise ValueError(f"a tile of {int(npx.max())} pixels exceeds the 2^32 - 1 pixels one tile may hold; use a smaller tile_size")
 
 
+RUN_DTYPE = np.dtype([("tile", "<i8"), ("first_frame", "<i8"), ("n_frames", "<i8"), ("byte_offset", "<i8"), ("byte_length", "<i8")])
+
+
+def window_frames(tiles: np.ndarray, window, blocksize: int, frame_bytes=None) -> np.ndarray:
+    """The frames a pixel window needs: one run per tile that intersects it (RUN_DTYPE records, in tile order).
+
+    tiles: TILE_DTYPE records in image coordinates; window: (col_off, row_off, width, height) in image coordinates.  A tile's
+    samples are its pixels in row-major order, so the visible ones lie between sample y0*w + x0 (first visible row, first
+    visible column) and (y1-1)*w + x1-1; the run is every frame from the one holding the first to the one holding the last.
+    frame_bytes (optional): per tile, the byte size of each of its frames (the "frbI" seek index); byte_offset / byte_length
+    of the run then give where its frames sit behind the stream's first frame.  Without it they are -1."""
+    col0, row0, width, height = (int(v) for v in window)
+    out = []
+    for i, t in enumerate(tiles):
+        r, c, h, w = int(t["row_off"]), int(t["col_off"]), int(t["h"]), int(t["w"])
+        y0, y1 = max(row0 - r, 0), min(row0 + height - r, h)
+        x0, x1 = max(col0 - c, 0), min(col0 + width - c, w)
+        if y0 >= y1 or x0 >= x1:
+            continue
+        f0 = (y0 * w + x0) // blocksize
+        f1 = ((y1 - 1) * w + x1 - 1) // blocksize + 1
+        off = length = -1
+        if frame_bytes is not None:
+            fb = np.asarray(frame_bytes[i], dtype=np.int64)
+            off, length = int(fb[:f0].sum()), int(fb[f0:f1].sum())
+        out.append((i, f0, f1 - f0, off, length))
+    return np.array(out, dtype=RUN_DTYPE)
+
+
+def bbox_to_window(transform, width: int, height: int, bbox) -> Tuple[int, int, int, int]:
+    """(xmin, ymin, xmax, ymax) in the raster's coordinates -> pixel window (col_off, row_off, width, height): the offsets
+    are floored, the far edges ceiled, and the result clipped to the raster.  ValueError when nothing is left."""
+    import math
+    a, b, c, d, e, f = (float(v) for v in transform[:6])
+    if b != 0.0 or d != 0.0 or a == 0.0 or e == 0.0:
+        raise ValueError("bbox reads need a north-up transform without rotation")
+    xmin, ymin, xmax, ymax = (float(v) for v in bbox)
+    cx = sorted(((xmin - c) / a, (xmax - c) / a))
+    ry = sorted(((ymin - f) / e, (ymax - f) / e))
+    c0, c1 = max(math.floor(cx[0]), 0), min(math.ceil(cx[1]), int(width))
+    r0, r1 = max(math.floor(ry[0]), 0), min(math.ceil(ry[1]), int(height))
+    if c1 <= c0 or r1 <= r0:
+        raise ValueError(f"bbox {tuple(bbox)} does not intersect the raster")
+    return c0, r0, c1 - c0, r1 - r0
+
+
 def _stream_ptr() -> int:
     return torch.cuda.current_stream().cuda_stream
 
@@ -586,6 +632,116 @@ class Engine:
             self._two_launch = True                  # offsets did not arrive inside the fused launch: separate skim launch from now on
             return self.decode_tiles(data, byte_offsets, byte_lengths, tiles, sample_rates, minmax, scale, out, bps, blocksize, verify_crc,
                                      fused, index)
+        return status
+
+    def decode_window(self, data: torch.Tensor, byte_offsets: np.ndarray, byte_lengths: np.ndarray, tiles: np.ndarray,
+                      sample_rates: np.ndarray, minmax: np.ndarray, scale: float, window, out: torch.Tensor, bps: int,
+                      blocksize: int = 4096, index=None, runs_only: bool = False, verify_crc: bool = True,
+                      fused: Optional[bool] = None) -> np.ndarray:
+        """The pixels of `window` (col_off, row_off, width, height, image coordinates) from the frames of the tiles that
+        cover it (image coordinates) -> the (bands, height, width) device array `out`.  Only the frames each tile's part of
+        the window needs are decoded (window_frames).  Returns the status words; status[3] counts the decoded frames.
+        byte_offsets / byte_lengths: where each tile's frames are in `data` -- all of them, or with `runs_only` only the
+        run's frames (a partial read; then the seek index is required, and a rejected index is reported in the status words
+        instead of falling back to a scan, which would need every frame).  index: (frame_bytes, sub_bitoff) of all the
+        tiles' frames in tile order (host arrays), or None (scan path).  `fused` as decode_tiles."""
+        bands = out.shape[0]
+        col0, row0, width, height = (int(v) for v in window)
+        if tuple(out.shape[1:]) != (height, width):
+            raise ValueError("out must have the window's shape")
+        n_samples = tiles["h"].astype(np.int64) * tiles["w"].astype(np.int64)
+        _check_tile_sizes(n_samples)
+        frames_all = (n_samples + blocksize - 1) // blocksize
+        fstart = np.concatenate([[0], np.cumsum(frames_all)])
+        if index is not None and index[0] is not None and (bands == 1 or index[1] is not None):
+            fb_all = np.asarray(index[0]).view(np.uint32).reshape(-1)
+            sb_all = np.asarray(index[1]).view(np.uint32).reshape(-1) if bands > 1 else None
+            if fb_all.size != fstart[-1] or (sb_all is not None and sb_all.size != fstart[-1] * bands):
+                fb_all = sb_all = None
+        else:
+            fb_all = sb_all = None
+        if runs_only and fb_all is None:
+            raise ValueError("decode_window(runs_only=True) needs the tiles' seek index")
+        runs = window_frames(tiles, window, blocksize,
+                             None if fb_all is None else [fb_all[fstart[i]:fstart[i + 1]] for i in range(len(tiles))])
+        if len(runs) == 0:
+            raise ValueError(f"window {tuple(window)} covers no tile")
+        sel = runs["tile"]
+        n_runs = len(runs)
+        dt = str(out.dtype).replace("torch.", "")
+        if fused is None:          # the rule decode_tiles measured: the exact integer form fused, the fp64 formula two-step
+            fused = bps == 16 and dt in ("uint8", "int8", "uint16", "int16") and float(scale) == 32767.0
+        two_step = bands == 2 or not fused
+        run_n = np.minimum((runs["first_frame"] + runs["n_frames"]) * blocksize, n_samples[sel]) - runs["first_frame"] * blocksize
+        st = np.zeros(n_runs, dtype=nat.WINDOW_STREAM_DTYPE)
+        st["total_samples"] = n_samples[sel]
+        st["sample_rate"] = np.asarray(sample_rates)[sel]
+        st["first_frame"] = runs["first_frame"]
+        st["n_frames"] = runs["n_frames"]
+        fbase = np.zeros(n_runs, dtype=np.int64)
+        np.cumsum(runs["n_frames"][:-1], out=fbase[1:])
+        st["frame_base"] = fbase
+        abase = np.zeros(n_runs, dtype=np.int64)
+        np.cumsum(run_n[:-1] * bands, out=abase[1:])
+        st["audio_base"] = abase
+        total_frames = int(runs["n_frames"].sum())
+        idx_host = None
+        if fb_all is not None:
+            parts_fb = [fb_all[fstart[t] + f0:fstart[t] + f0 + n] for t, f0, n in zip(sel, runs["first_frame"], runs["n_frames"])]
+            parts_sb = [sb_all[(fstart[t] + f0) * bands:(fstart[t] + f0 + n) * bands]
+                        for t, f0, n in zip(sel, runs["first_frame"], runs["n_frames"])] if bands > 1 else None
+            idx_host = (np.concatenate(parts_fb), np.concatenate(parts_sb) if bands > 1 else None)
+        offs = np.asarray(byte_offsets, dtype=np.int64)[sel]
+        lens = np.asarray(byte_lengths, dtype=np.int64)[sel]
+        with torch.cuda.device(self.device):
+            s = _stream_ptr()
+            stage = np.zeros(n_runs * 32, dtype=np.uint8)
+            stage[: n_runs * 16] = np.ascontiguousarray(tiles[sel]).view(np.uint8)
+            stage[n_runs * 16:] = np.ascontiguousarray(np.asarray(minmax, dtype=np.float64).reshape(-1, 2)[sel]).reshape(-1).view(np.uint8)
+            d_stage = self._upload(stage)
+            d_status = torch.zeros(8, dtype=torch.int32, device=self.device)
+            idx = None if idx_host is None else self._index_on_device(idx_host, total_frames, bands)
+            audio = self._buf("win_audio", int(run_n.sum()) * bands * 4) if two_step else None
+            win = nat.Tile(row0, col0, height, width)
+            status = None
+            for max_order, use_idx in ((12, True), (32, True), (12, False), (32, False)):
+                if use_idx and idx is None:
+                    continue
+                if not use_idx and runs_only:
+                    break                            # the scan path needs every frame of the streams: the caller decides
+                if use_idx:
+                    st["byte_offset"] = offs if runs_only else offs + runs["byte_offset"]
+                    st["byte_length"] = lens if runs_only else runs["byte_length"]
+                else:
+                    st["byte_offset"], st["byte_length"] = offs, lens
+                p = nat.DecodeParams(n_runs, bands, bps, blocksize, (1 if verify_crc else 0) | (2 if self._two_launch else 0), max_order)
+                ws_bytes = C.c_size_t(0)
+                nat.check(self.L.frb_decode_workspace_size(C.byref(p), total_frames, C.byref(ws_bytes)), "frb_decode_workspace_size")
+                ws = self._buf("dec_ws", ws_bytes.value)
+                nat.check(self.L.frb_decode_window(C.byref(p), st.ctypes.data, data.data_ptr(), total_frames,
+                                                   idx[0].data_ptr() if use_idx else None, idx[1].data_ptr() if use_idx else None,
+                                                   d_stage.data_ptr(), d_stage.data_ptr() + n_runs * 16, float(scale), win,
+                                                   audio.data_ptr() if two_step else out.data_ptr(), -1 if two_step else nat.DTYPE_CODES[dt],
+                                                   ws.data_ptr(), ws.numel(), d_status.data_ptr(), s), "frb_decode_window")
+                status = self._download(d_status, np.int32, 8).astype(np.int64)      # (synchronises: d_stage stays alive)
+                if status[6]:
+                    raise nat.NativeError(nat.ERR_INVALID_ARG, "frb_decode_window",
+                                          f"{int(status[6])} tile(s) do not hold as many pixels as their stream has samples")
+                if use_idx and (status[0] or status[1] or status[2]):
+                    idx = None                       # the index does not describe these bytes: decode again by scanning
+                    continue
+                if status[4] == 0:
+                    break
+            if status[5] and not self._two_launch:
+                self._two_launch = True              # offsets did not arrive inside the fused launch: separate skim launch from now on
+                return self.decode_window(data, byte_offsets, byte_lengths, tiles, sample_rates, minmax, scale, window, out, bps,
+                                          blocksize, index, runs_only, verify_crc, fused)
+            if two_step and not (status[0] or status[1] or status[2] or status[4] or status[5]):
+                d_st = self._upload(st)
+                nat.check(self.L.frb_denormalize_window(audio.data_ptr(), d_st.data_ptr(), n_runs, blocksize, d_stage.data_ptr(),
+                                                        d_stage.data_ptr() + n_runs * 16, float(scale), win, out.data_ptr(),
+                                                        nat.DTYPE_CODES[dt], bands, s), "frb_denormalize_window")
+                torch.cuda.current_stream().synchronize()
         return status
 
     def decode_tiles_host(self, host_payload: torch.Tensor, byte_offsets: np.ndarray, byte_lengths: np.ndarray, tiles: np.ndarray,

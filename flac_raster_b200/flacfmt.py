@@ -167,3 +167,43 @@ def parse_header(data: bytes | memoryview) -> FlacHeader:
     if si is None:
         raise ValueError("missing STREAMINFO")
     return FlacHeader(si, tags, vendor, pos, apps)
+
+
+def read_header(read, first: int = 1 << 16) -> FlacHeader:
+    """parse_header for a stream that is read piece by piece: read(start, n) returns up to n bytes from `start` (a local
+    file or HTTP range requests).  A first piece of `first` bytes; a block that reaches beyond it is read in one more piece
+    together with the header of the block behind it.  The body of a PADDING block at the end of the chain is not read."""
+    buf = bytearray(read(0, first))
+    if len(buf) < 8 or bytes(buf[:4]) != b"fLaC":
+        raise ValueError("not a FLAC stream (missing fLaC marker)")
+
+    def have(end: int) -> bool:
+        if end > len(buf):
+            buf.extend(read(len(buf), end - len(buf)))
+        return end <= len(buf)
+
+    pos, last, si, tags, vendor, apps = 4, False, None, {}, "", {}
+    while not last:
+        if not have(pos + 4):
+            raise ValueError("truncated metadata")
+        h = buf[pos]
+        last = bool(h & 0x80)
+        btype = h & 0x7F
+        blen = int.from_bytes(bytes(buf[pos + 1:pos + 4]), "big")
+        pos += 4
+        if btype == 127:
+            raise ValueError("invalid metadata block type")
+        if btype in (BLOCK_STREAMINFO, BLOCK_VORBIS_COMMENT, BLOCK_APPLICATION) or not last:
+            if not have(pos + blen + (0 if last else 4)) and not have(pos + blen):
+                raise ValueError("truncated metadata block")
+            body = bytes(buf[pos:pos + blen])
+            if btype == BLOCK_STREAMINFO:
+                si = StreamInfo.unpack(body)
+            elif btype == BLOCK_VORBIS_COMMENT:
+                vendor, tags = unpack_vorbis_comment(body)
+            elif blen >= 4:
+                apps[body[:4]] = body[4:]
+        pos += blen
+    if si is None:
+        raise ValueError("missing STREAMINFO")
+    return FlacHeader(si, tags, vendor, pos, apps)

@@ -706,6 +706,84 @@ class SpatialFLACStreamer:
             return []
         return self._decode(frames)
 
+    def read_bbox(self, xmin, ymin, xmax, ymax):
+        """One mosaic of the pixels inside a bbox -> ((bands, h, w) array in the original dtype, metadata with its window,
+        transform and bounds).  The pixel window floors the bbox's near edges and ceils its far edges, clipped to the raster
+        (ValueError when the bbox misses it).  The tiles that intersect the window are fetched like get_tiles_by_bbox, and one
+        decode launch writes each tile's visible part straight into the mosaic, decoding only the frames that cover it."""
+        import torch
+        from . import _native as nat
+        from .converter import _raise_for_status, affine9
+        from .engine import TORCH_DTYPES, bbox_to_window, default_engine
+
+        frames = self.spatial_index.frames
+        H = max(int(f.window.row_off) + int(f.window.height) for f in frames)
+        W = max(int(f.window.col_off) + int(f.window.width) for f in frames)
+        tr = (self.metadata or {}).get("transform") or self.spatial_index.transform or None
+        t6 = tuple(float(v) for v in tr[:6]) if tr else (1.0, 0.0, 0.0, 0.0, -1.0, 0.0)     # _tile_bbox's default
+        col0, row0, width, height = bbox_to_window(t6, W, H, (xmin, ymin, xmax, ymax))
+        sel = [f for f in frames if int(f.window.col_off) < col0 + width and int(f.window.col_off) + int(f.window.width) > col0
+               and int(f.window.row_off) < row0 + height and int(f.window.row_off) + int(f.window.height) > row0]
+        stage, nbytes, starts = self._read_tiles_pinned(sel)
+        view = memoryview(stage.numpy())
+        n = len(sel)
+        tiles = np.zeros(n, dtype=nat.TILE_DTYPE)
+        offs, lens = np.zeros(n, dtype=np.int64), np.zeros(n, dtype=np.int64)
+        rates = np.zeros(n, dtype=np.uint32)
+        minmax = np.zeros((n, 2), dtype=np.float64)
+        fb, sb = [], []
+        md0 = None
+        for i, f in enumerate(sel):
+            blob = view[int(starts[i]):int(starts[i]) + f.byte_size]
+            h = flacfmt.parse_header(blob)
+            md = parse_metadata_tags(h.tags)
+            if self.metadata is None and not (md and int(md.get("width", 0)) * int(md.get("height", 0)) == int(f.window.width) * int(f.window.height)):
+                md = self._legacy_tile_metadata(f, h.streaminfo)        # reference-written legacy file (see _decode)
+            if not md:
+                raise ValueError("No metadata found in FLAC file or sidecar file")
+            si = h.streaminfo
+            if md0 is None:
+                md0, si0 = md, si
+            elif (si.channels, si.bits_per_sample, si.max_blocksize, md["dtype"]) != (si0.channels, si0.bits_per_sample, si0.max_blocksize, md0["dtype"]):
+                raise ValueError("tiles of one mosaic must share channels, bits per sample, blocksize and dtype")
+            if int(md["width"]) != int(f.window.width) or int(md["height"]) != int(f.window.height):
+                raise ValueError(f"tile {f.frame_id}: its tags do not match its window in the index")
+            tiles[i] = (int(f.window.row_off), int(f.window.col_off), int(f.window.height), int(f.window.width))
+            offs[i], lens[i] = int(starts[i]) + h.first_frame_offset, f.byte_size - h.first_frame_offset
+            rates[i] = si.sample_rate
+            minmax[i] = (md["data_min"], md["data_max"])
+            if fb is not None:
+                blk = h.applications.get(flacfmt.SEEK_INDEX_ID)
+                nf = (int(f.window.width) * int(f.window.height) + si.max_blocksize - 1) // si.max_blocksize
+                got = flacfmt.unpack_seek_index(blk, si.channels, si.max_blocksize, nf) if blk else None
+                if got is None:
+                    fb = sb = None
+                else:
+                    fb.append(got[0])
+                    sb.append(got[1])
+        bands, bps, blocksize = si0.channels, si0.bits_per_sample, si0.max_blocksize
+        index = (np.concatenate(fb), np.concatenate(sb) if bands > 1 else None) if fb else None
+        scale = 32767.0 if bps == 16 else 8388607.0                  # decode default by audio width (converter.py:220-229)
+        dtype = np.dtype(md0["dtype"])
+        eng = default_engine()
+        stage[nbytes:nbytes + 64].zero_()
+        data = eng._buf("dec_data", nbytes + 64)[:nbytes + 64]
+        data.copy_(stage[:nbytes + 64], non_blocking=True)
+        out = torch.empty((bands, height, width), dtype=TORCH_DTYPES[str(dtype)], device=eng.device)
+        status = eng.decode_window(data, offs, lens, tiles, rates, minmax, scale, (col0, row0, width, height), out, bps, blocksize,
+                                   index=index)
+        _raise_for_status(status)
+        wt = window_transform(t6, col0, row0)
+        left, top = wt[2], wt[5]
+        meta = {
+            "crs": (self.metadata or {}).get("crs", md0.get("crs", "")), "width": width, "height": height, "count": bands,
+            "dtype": str(dtype), "nodata": md0.get("nodata"), "transform": affine9(wt) if tr else None,
+            "bounds": {"left": left, "bottom": top + height * wt[4], "right": left + width * wt[0], "top": top},
+            "window": {"col_off": col0, "row_off": row0, "width": width, "height": height},
+            "tiles": [f.frame_id for f in sel], "frames_decoded": int(status[3]),
+        }
+        return out.cpu().numpy(), meta
+
     def get_center_tile(self):
         """cli.py:250-262: tile whose centroid is nearest the centroid of the union of bboxes."""
         fr = self.spatial_index.frames

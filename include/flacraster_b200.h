@@ -268,6 +268,53 @@ int frb_decode_tiles_indexed(const frb_decode_params *p, const frb_decode_stream
                              void *d_raster, int dtype, uint32_t bands, uint32_t H, uint32_t W,
                              void *d_workspace, size_t workspace_bytes, uint32_t *d_status, void *stream);
 
+/* Windowed read: a pixel window of a raster whose tiles are FLAC streams, decoding only the frames that cover it.
+ * The sample order of a tile is row-major, so the samples of tile t that fall inside the window lie between its first
+ * and its last visible pixel: a run of consecutive frames [first_frame, first_frame + n_frames) per stream.  A run is
+ * decoded as a stream of its own (the indexed path never compares a frame's coded number with its position; the scan
+ * path uses the coded numbers to find the run's frames and the frame behind it).
+ *   byte_offset / byte_length: indexed path (d_frame_bytes != NULL): the bytes of the run's frames only; scan path: the
+ *                              bytes of ALL the stream's frames (the scan finds the run's frames by number)
+ *   total_samples:             samples per channel of the whole stream (h*w of its tile)
+ *   audio_base:                dtype -1 only: index into d_out of the run's channel 0, first sample; the run's samples
+ *                              per channel are min(n_frames * blocksize, total_samples - first_frame * blocksize)
+ *   frame_base:                exclusive scan of n_frames (the run's frames in d_frame_bytes / d_sub_bitoff) */
+typedef struct frb_window_stream {
+    uint64_t byte_offset;
+    uint64_t byte_length;
+    uint64_t total_samples;
+    int64_t  audio_base;
+    uint32_t sample_rate;
+    uint32_t frame_base;
+    uint32_t first_frame;
+    uint32_t n_frames;
+} frb_window_stream;
+
+/* Decodes the frame runs of h_streams and writes the pixels of stream i (tile d_tiles[i], image coordinates) that lie
+ * inside `window` (image coordinates; row_off, col_off, h, w) to d_out, a (bands, window.h, window.w) array of `dtype`:
+ * pixel (y, x) of the image lands at d_out[c, y - window.row_off, x - window.col_off].  Pixels of a run outside the window
+ * are decoded (the frames have to be) but not stored.  The values are bit-identical to frb_decode_tiles (same integer
+ * form, same fp64 tie path).  Tiles may overlap the window partly or not at all.
+ * d_frame_bytes (total_frames entries: the runs' frame sizes, run after run) and d_sub_bitoff (total_frames * channels)
+ * select the indexed path; both NULL select the scan path.  total_frames = sum of n_frames.
+ * dtype -1: no pixels, d_out receives the runs' int32 planar audio at audio_base (two-channel streams, whose frames may
+ * be mid/side coded, and the dtypes whose mapping runs faster as a kernel of its own): then frb_denormalize_window.
+ * Otherwise two-channel streams return FRB_ERR_UNSUPPORTED.
+ * Workspace: frb_decode_workspace_size(p, total_frames).  Status words as frb_decode_batch; frames_decoded counts the run
+ * frames, tiles_rejected counts streams whose tile does not hold total_samples pixels.  Only the decoded frames are
+ * validated: a damaged frame outside the runs is not seen. */
+int frb_decode_window(const frb_decode_params *p, const frb_window_stream *h_streams,
+                      const uint8_t *d_bytes, uint64_t total_frames,
+                      const uint32_t *d_frame_bytes, const uint32_t *d_sub_bitoff,
+                      const frb_tile *d_tiles, const double *d_minmax, double scale, frb_tile window,
+                      void *d_out, int dtype, void *d_workspace, size_t workspace_bytes, uint32_t *d_status, void *stream);
+
+/* The pixels of the window from the int32 audio frb_decode_window wrote with dtype -1 (same mapping as
+ * frb_denormalize_tiles).  d_streams: the stream table of that call copied to the device; d_out as frb_decode_window. */
+int frb_denormalize_window(const int32_t *d_audio, const frb_window_stream *d_streams, uint32_t n_tiles, uint32_t blocksize,
+                           const frb_tile *d_tiles, const double *d_minmax, double scale, frb_tile window,
+                           void *d_out, int dtype, uint32_t bands, void *stream);
+
 /* Frame discovery for a stream of unknown length (FileDecoder on a file
  * whose STREAMINFO total_samples is 0 and no tags are known).  Synchronous.
  * Returns the number of frames and the total samples per channel. */
