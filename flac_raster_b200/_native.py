@@ -53,6 +53,16 @@ class DecodeParams(C.Structure):
                 ("blocksize", C.c_uint32), ("verify_crc16", C.c_uint32), ("reserved", C.c_uint32)]
 
 
+# the eight status words every decode call writes (d_status of frb_decode_batch), in order; the eighth is always 0
+(ST_FRAMES_MISSING, ST_CRC16_ERRORS, ST_PARSE_ERRORS, ST_FRAMES_DECODED, ST_LPC_ORDER_ABOVE_12, ST_OFFSET_WAIT_TIMEOUTS,
+ ST_TILES_REJECTED, ST_RESERVED) = range(8)
+
+
+def status_damaged(status) -> bool:
+    """Frames missing, a CRC-16 mismatch or a parse error: the bytes (or their seek index) do not hold the frames asked for."""
+    return bool(status[ST_FRAMES_MISSING] or status[ST_CRC16_ERRORS] or status[ST_PARSE_ERRORS])
+
+
 TILE_HEADER_DTYPE = np.dtype([
     ("first_frame_offset", "<u4"), ("sample_rate", "<u4"), ("channels", "<u4"), ("bps", "<u4"), ("min_blocksize", "<u4"),
     ("max_blocksize", "<u4"), ("width", "<u4"), ("height", "<u4"), ("count", "<u4"), ("dtype", "<i4"), ("flags", "<u4"),

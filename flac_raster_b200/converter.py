@@ -246,7 +246,7 @@ class RasterFLACConverter:
             if len(blob) == int(run["byte_length"]):
                 status = eng.decode_window(to_device(blob), np.zeros(1, np.int64), np.array([len(blob)]), tiles, rates, minmax,
                                            scale, window, out, bps, blocksize, index=index, runs_only=True)
-        if status is None or status[0] or status[1] or status[2]:
+        if status is None or nat.status_damaged(status):
             # no index, or one that does not describe the frames: every frame is needed to find the window's by scanning
             blob = read(hdr.first_frame_offset, -1) if not is_remote_url(src) else rf.read_all()[hdr.first_frame_offset:]
             status = eng.decode_window(to_device(blob), np.zeros(1, np.int64), np.array([len(blob)]), tiles, rates, minmax,
@@ -261,7 +261,7 @@ class RasterFLACConverter:
                      "bounds": {"left": left, "bottom": top + height * (t6[4] if t6 else -1.0),
                                 "right": left + width * (t6[0] if t6 else 1.0), "top": top},
                      "window": {"col_off": col_off, "row_off": row_off, "width": width, "height": height},
-                     "frames_decoded": int(status[3])})
+                     "frames_decoded": int(status[nat.ST_FRAMES_DECODED])})
         return res, meta
 
     # kept for signature compatibility with the reference (converter.py:263, :329)
@@ -532,12 +532,13 @@ def full_tiles_first(widths, heights, channels: int):
 
 
 def _raise_for_status(status):
-    if status[5]:
+    from . import _native as nat
+    if status[nat.ST_OFFSET_WAIT_TIMEOUTS]:
         raise RuntimeError("decode kernel timed out waiting for a subframe offset")
-    if status[0] or status[2]:
-        raise ValueError(f"malformed FLAC stream (missing frames={status[0]}, parse errors={status[2]})")
-    if status[1]:
-        raise ValueError(f"FLAC frame CRC-16 mismatch in {status[1]} frame(s)")
+    if status[nat.ST_FRAMES_MISSING] or status[nat.ST_PARSE_ERRORS]:
+        raise ValueError(f"malformed FLAC stream (missing frames={status[nat.ST_FRAMES_MISSING]}, parse errors={status[nat.ST_PARSE_ERRORS]})")
+    if status[nat.ST_CRC16_ERRORS]:
+        raise ValueError(f"FLAC frame CRC-16 mismatch in {status[nat.ST_CRC16_ERRORS]} frame(s)")
 
 
 def _copy_tiles_out(host_out, rows0, heights, widths):

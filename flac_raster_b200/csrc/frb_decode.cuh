@@ -321,24 +321,48 @@ static int check_decode_args(const frb_decode_params *p, const void *h_streams, 
     return FRB_OK;
 }
 
+// The sink of a decode to planar int32 audio.
+static SinkCfg audio_sink() { SinkCfg sink; memset(&sink, 0, sizeof sink); sink.dtype = -1; return sink; }
+
+// The sink of a decode straight into a (bands, H, W) raster of `dtype` at `out`.  frb_decode_tiles and frb_decode_window
+// both take it from here, which is what keeps a window's pixels bit-identical to those of a whole decode.
+static SinkCfg raster_sink(int dtype, double scale, const frb_tile *d_tiles, const double *d_minmax, void *out, uint32_t H, uint32_t W) {
+    static const uint32_t esz[8] = {1, 1, 2, 2, 4, 4, 4, 8};
+    SinkCfg sink = audio_sink();
+    sink.dtype = dtype; sink.esize = esz[dtype]; sink.H = H; sink.W = W; sink.tiles = d_tiles; sink.minmax = d_minmax;
+    sink.raster = (uint8_t *)out; sink.scale = scale; sink.rcp = 1.0 / scale;
+    sink.fast = (scale == 32767.0 || scale == 8388607.0 || scale == 2147483647.0) ? 1 : 0;
+    sink.intpath = (dtype <= FRB_I16 && scale == 32767.0) ? 1 : 0;      // integer min/max, range < 2^16, |audio| <= 32767
+    return sink;
+}
+
+// One entry of the device stream table: frames [first_frame, first_frame + n_frames) of a stream of total_samples samples,
+// which must lie inside the stream.  `frames`: the frames of the entries before it, which frame_base must equal.
+static int dec_stream(const frb_decode_params *p, uint64_t byte_offset, uint64_t byte_length, uint64_t total_samples,
+                      int64_t audio_base, uint32_t sample_rate, uint32_t frame_base, uint32_t first_frame, uint64_t n_frames,
+                      uint64_t &frames, DecStreamDev &d) {
+    const uint64_t all = (total_samples + p->blocksize - 1) / p->blocksize;
+    if (all > 0xFFFFFFFFull || first_frame + n_frames > all || frame_base != frames) return FRB_ERR_INVALID_ARG;
+    const uint64_t s0 = (uint64_t)first_frame * p->blocksize, s1 = (first_frame + n_frames) * p->blocksize;
+    d.byte_offset = byte_offset; d.byte_length = byte_length; d.n_samples = (s1 < total_samples ? s1 : total_samples) - s0;
+    d.audio_base = audio_base; d.sample_rate = sample_rate; d.frame_base = frame_base; d.n_frames = (uint32_t)n_frames;
+    d.first_frame = first_frame; d.total_samples = total_samples; d.total_frames = (uint32_t)all; d.pad = 0;
+    frames += n_frames;
+    return FRB_OK;
+}
+
 static int decode_batch_impl(const frb_decode_params *p, const frb_decode_stream *h_streams,
                              const uint8_t *d_bytes, uint64_t total_frames, int32_t *d_audio,
                              void *d_workspace, size_t workspace_bytes, uint32_t *d_status, void *stream, const SinkCfg &sink,
                              const uint32_t *d_frame_bytes = nullptr, const uint32_t *d_index_bitoff = nullptr) {
     FRB_TRY(check_decode_args(p, h_streams, d_bytes, total_frames, d_audio, d_workspace, d_status, sink, d_frame_bytes, d_index_bitoff));
-    // stream table (host -> device). Pageable source: staged by the runtime before return.
+    // stream table (host -> device), every stream whole. Pageable source: staged by the runtime before return.
     std::vector<DecStreamDev> hs(p->n_streams);
     uint64_t frames = 0;
     for (uint32_t i = 0; i < p->n_streams; i++) {
         const frb_decode_stream &a = h_streams[i];
-        DecStreamDev d;
-        d.byte_offset = a.byte_offset; d.byte_length = a.byte_length; d.n_samples = a.n_samples;
-        d.audio_base = a.audio_base; d.sample_rate = a.sample_rate; d.frame_base = a.frame_base;
-        d.n_frames = (uint32_t)((a.n_samples + p->blocksize - 1) / p->blocksize);
-        d.first_frame = 0; d.total_samples = d.n_samples; d.total_frames = d.n_frames; d.pad = 0;
-        if (a.frame_base != frames) return FRB_ERR_INVALID_ARG;
-        frames += d.n_frames;
-        hs[i] = d;
+        FRB_TRY(dec_stream(p, a.byte_offset, a.byte_length, a.n_samples, a.audio_base, a.sample_rate, a.frame_base, 0,
+                           (a.n_samples + p->blocksize - 1) / p->blocksize, frames, hs[i]));
     }
     if (frames != total_frames) return FRB_ERR_INVALID_ARG;
     return decode_streams_impl(p, hs, d_bytes, total_frames, d_audio, d_workspace, workspace_bytes, d_status, stream, sink,
@@ -488,10 +512,8 @@ static int decode_streams_impl(const frb_decode_params *p, const std::vector<Dec
 extern "C" int frb_decode_batch(const frb_decode_params *p, const frb_decode_stream *h_streams,
                                 const uint8_t *d_bytes, uint64_t total_frames, int32_t *d_audio,
                                 void *d_workspace, size_t workspace_bytes, uint32_t *d_status, void *stream) {
-    frb::SinkCfg sink;
-    memset(&sink, 0, sizeof sink);
-    sink.dtype = -1;
-    return frb::decode_batch_impl(p, h_streams, d_bytes, total_frames, d_audio, d_workspace, workspace_bytes, d_status, stream, sink);
+    return frb::decode_batch_impl(p, h_streams, d_bytes, total_frames, d_audio, d_workspace, workspace_bytes, d_status, stream,
+                                  frb::audio_sink());
 }
 
 static int frb_decode_tiles_impl(const frb_decode_params *p, const frb_decode_stream *h_streams,
@@ -506,15 +528,8 @@ static int frb_decode_tiles_impl(const frb_decode_params *p, const frb_decode_st
     // two-channel streams may carry left/side, side/right or mid/side frames, whose samples only exist after both
     // subframes have been decoded: those go through frb_decode_batch + frb_denormalize_tiles
     if (p->channels == 2) return FRB_ERR_UNSUPPORTED;
-    static const uint32_t esz[8] = {1, 1, 2, 2, 4, 4, 4, 8};
-    SinkCfg sink;
-    memset(&sink, 0, sizeof sink);
-    sink.dtype = dtype; sink.esize = esz[dtype]; sink.H = H; sink.W = W; sink.tiles = d_tiles; sink.minmax = d_minmax;
-    sink.raster = (uint8_t *)d_raster; sink.scale = scale; sink.rcp = 1.0 / scale;
-    sink.fast = (scale == 32767.0 || scale == 8388607.0 || scale == 2147483647.0) ? 1 : 0;
-    sink.intpath = (dtype <= FRB_I16 && scale == 32767.0) ? 1 : 0;      // integer min/max, range < 2^16, |audio| <= 32767
-    return decode_batch_impl(p, h_streams, d_bytes, total_frames, nullptr, d_workspace, workspace_bytes, d_status, stream, sink,
-                             d_frame_bytes, d_sub_bitoff);
+    return decode_batch_impl(p, h_streams, d_bytes, total_frames, nullptr, d_workspace, workspace_bytes, d_status, stream,
+                             raster_sink(dtype, scale, d_tiles, d_minmax, d_raster, H, W), d_frame_bytes, d_sub_bitoff);
 }
 
 extern "C" int frb_decode_tiles(const frb_decode_params *p, const frb_decode_stream *h_streams,
@@ -542,11 +557,8 @@ extern "C" int frb_decode_batch_indexed(const frb_decode_params *p, const frb_de
                                         const uint32_t *d_frame_bytes, const uint32_t *d_sub_bitoff, int32_t *d_audio,
                                         void *d_workspace, size_t workspace_bytes, uint32_t *d_status, void *stream) {
     if (!d_frame_bytes || !d_sub_bitoff) return FRB_ERR_INVALID_ARG;
-    frb::SinkCfg sink;
-    memset(&sink, 0, sizeof sink);
-    sink.dtype = -1;
-    return frb::decode_batch_impl(p, h_streams, d_bytes, total_frames, d_audio, d_workspace, workspace_bytes, d_status, stream, sink,
-                                  d_frame_bytes, d_sub_bitoff);
+    return frb::decode_batch_impl(p, h_streams, d_bytes, total_frames, d_audio, d_workspace, workspace_bytes, d_status, stream,
+                                  frb::audio_sink(), d_frame_bytes, d_sub_bitoff);
 }
 
 extern "C" int frb_decode_window(const frb_decode_params *p, const frb_window_stream *h_streams,
@@ -558,34 +570,17 @@ extern "C" int frb_decode_window(const frb_decode_params *p, const frb_window_st
     if (!p || !d_out || dtype < -1 || dtype > FRB_F64) return FRB_ERR_INVALID_ARG;
     if (dtype >= 0 && (!d_tiles || !d_minmax || !(scale > 0.0) || window.h == 0 || window.w == 0)) return FRB_ERR_INVALID_ARG;
     if (dtype >= 0 && p->channels == 2) return FRB_ERR_UNSUPPORTED;       // mid/side frames: dtype -1 + frb_denormalize_window
-    SinkCfg sink;
-    memset(&sink, 0, sizeof sink);
-    sink.dtype = -1;
-    if (dtype >= 0) {
-        static const uint32_t esz[8] = {1, 1, 2, 2, 4, 4, 4, 8};
-        sink.dtype = dtype; sink.esize = esz[dtype]; sink.H = window.h; sink.W = window.w; sink.tiles = d_tiles; sink.minmax = d_minmax;
-        sink.raster = (uint8_t *)d_out; sink.scale = scale; sink.rcp = 1.0 / scale;
-        sink.fast = (scale == 32767.0 || scale == 8388607.0 || scale == 2147483647.0) ? 1 : 0;
-        sink.intpath = (dtype <= FRB_I16 && scale == 32767.0) ? 1 : 0;
-        sink.window = 1; sink.win_row = window.row_off; sink.win_col = window.col_off;
-    }
+    SinkCfg sink = dtype >= 0 ? raster_sink(dtype, scale, d_tiles, d_minmax, d_out, window.h, window.w) : audio_sink();
+    if (dtype >= 0) { sink.window = 1; sink.win_row = window.row_off; sink.win_col = window.col_off; }
     int32_t *d_audio = dtype < 0 ? (int32_t *)d_out : nullptr;
     FRB_TRY(check_decode_args(p, h_streams, d_bytes, total_frames, d_audio, d_workspace, d_status, sink, d_frame_bytes, d_sub_bitoff));
     std::vector<DecStreamDev> hs(p->n_streams);
     uint64_t frames = 0;
     for (uint32_t i = 0; i < p->n_streams; i++) {
         const frb_window_stream &a = h_streams[i];
-        DecStreamDev d;
-        const uint64_t all = (a.total_samples + p->blocksize - 1) / p->blocksize;
-        if (a.n_frames == 0 || all > 0xFFFFFFFFull || (uint64_t)a.first_frame + a.n_frames > all || a.frame_base != frames)
-            return FRB_ERR_INVALID_ARG;
-        const uint64_t s0 = (uint64_t)a.first_frame * p->blocksize, s1 = (uint64_t)(a.first_frame + a.n_frames) * p->blocksize;
-        d.byte_offset = a.byte_offset; d.byte_length = a.byte_length;
-        d.n_samples = (s1 < a.total_samples ? s1 : a.total_samples) - s0;
-        d.audio_base = a.audio_base; d.sample_rate = a.sample_rate; d.frame_base = a.frame_base; d.n_frames = a.n_frames;
-        d.first_frame = a.first_frame; d.total_samples = a.total_samples; d.total_frames = (uint32_t)all; d.pad = 0;
-        frames += a.n_frames;
-        hs[i] = d;
+        if (a.n_frames == 0) return FRB_ERR_INVALID_ARG;
+        FRB_TRY(dec_stream(p, a.byte_offset, a.byte_length, a.total_samples, a.audio_base, a.sample_rate, a.frame_base,
+                           a.first_frame, a.n_frames, frames, hs[i]));
     }
     if (frames != total_frames) return FRB_ERR_INVALID_ARG;
     return decode_streams_impl(p, hs, d_bytes, total_frames, d_audio, d_workspace, workspace_bytes, d_status, stream, sink,

@@ -93,6 +93,65 @@ def bbox_to_window(transform, width: int, height: int, bbox) -> Tuple[int, int, 
     return c0, r0, c1 - c0, r1 - r0
 
 
+def _stream_table(byte_offsets, byte_lengths, n_samples, sample_rates, channels: int, blocksize: int):
+    """Whole streams as DECODE_STREAM_DTYPE records, and where each stream's frames start in the batch (n_streams + 1
+    entries, the last one the batch's frame count).  frame_base and audio_base are the exclusive scans of the streams'
+    frame and sample counts."""
+    n_samples = np.asarray(n_samples, dtype=np.int64)
+    fstart = np.zeros(len(n_samples) + 1, dtype=np.int64)
+    np.cumsum((n_samples + blocksize - 1) // blocksize, out=fstart[1:])
+    st = np.zeros(len(n_samples), dtype=nat.DECODE_STREAM_DTYPE)
+    st["byte_offset"] = byte_offsets
+    st["byte_length"] = byte_lengths
+    st["n_samples"] = n_samples
+    st["audio_base"][1:] = np.cumsum(n_samples[:-1] * channels)
+    st["sample_rate"] = sample_rates
+    st["frame_base"] = fstart[:-1]
+    return st, fstart
+
+
+def _index_fits(index, total_frames: int, channels: int) -> bool:
+    """Whether index = (frame_bytes, sub_bitoff) has the shape of the seek index of `total_frames` frames: one frame size per
+    frame and, for more than one channel, one subframe bit offset per subframe (sub_bitoff is not used for one channel)."""
+    def size(x):
+        return -1 if x is None else x.numel() if isinstance(x, torch.Tensor) else np.size(x)
+
+    return index is not None and size(index[0]) == total_frames and (channels == 1 or size(index[1]) == total_frames * channels)
+
+
+def _fused_default(bps: int, dtype: str, scale: float) -> bool:
+    """Whether decode_tiles and decode_window denormalise inside the decode launch when the caller does not say.  The fused
+    launch pays off where the pixel mapping is the exact integer form (8/16-bit rasters behind 16-bit audio).  Wider dtypes
+    need the fp64 formula per sample, which is cheaper in the bandwidth-bound mapping kernel than inside the issue-bound
+    decode kernel (C4 float32: 129 vs 97 GSamples/s), so they stay two-step."""
+    return bps == 16 and dtype in ("uint8", "int8", "uint16", "int16") and float(scale) == 32767.0
+
+
+def decode_ladder(attempt, has_index: bool, allow_scan: bool, where: str):
+    """The decodes every device decode call tries, which decide what a damaged, foreign or wrongly indexed stream turns into.
+    attempt(max_order, use_index) decodes once and returns the host status words; the status words of the last attempt are
+    returned.  Order: seek index at LPC order <= 12, index at order 32, sync scan at 12, scan at 32.  Index attempts need an
+    index, and damage under it drops it: the index does not describe the bytes, so decode again by scanning -- unless
+    `allow_scan` is False (the bytes hold only some frames of each stream), where the damaged words come back for the caller
+    to judge.  Rejected tiles raise NativeError: they are the caller's error, not the stream's."""
+    status = None
+    for max_order, use_index in ((12, True), (32, True), (12, False), (32, False)):
+        if use_index and not has_index:
+            continue
+        if not use_index and not allow_scan:
+            break
+        status = attempt(max_order, use_index)
+        if status[nat.ST_TILES_REJECTED]:
+            raise nat.NativeError(nat.ERR_INVALID_ARG, where, f"{int(status[nat.ST_TILES_REJECTED])} tile(s) do not hold as many "
+                                  "pixels as their stream has samples, or lie outside the raster")
+        if use_index and nat.status_damaged(status):
+            has_index = False
+            continue
+        if status[nat.ST_LPC_ORDER_ABOVE_12] == 0:
+            break
+    return status
+
+
 def _stream_ptr() -> int:
     return torch.cuda.current_stream().cuda_stream
 
@@ -140,7 +199,7 @@ class Engine:
         self._ws: dict[str, torch.Tensor] = {}
         # scan-path decode of multi-channel streams: False = skim CTAs inside the decode launch (in-order CTA dispatch assumed),
         # True = skim as its own launch.  Switched on for good the first time a decode thread reports that it gave up waiting
-        # for a subframe offset (status[5]): the device is shared or does not dispatch in order.
+        # for a subframe offset (ST_OFFSET_WAIT_TIMEOUTS): the device is shared or does not dispatch in order.  See _decode.
         self._two_launch = False
 
     # ---------------------------------------------------------------- helpers
@@ -474,46 +533,49 @@ class Engine:
                             np.concatenate([p.sample_rates for p in parts]), p0.channels, p0.bps, p0.bits_per_sample, p0.blocksize, fb, sb)
 
     # ------------------------------------------------------------------ decode
+    def _decode_params(self, n_streams: int, channels: int, bps: int, blocksize: int, verify_crc: bool, max_order: int,
+                       total_frames: int, ws_name: str):
+        """DecodeParams of one decode attempt in the engine's current launch mode, and its workspace."""
+        p = nat.DecodeParams(n_streams, channels, bps, blocksize, (1 if verify_crc else 0) | (2 if self._two_launch else 0), max_order)
+        ws_bytes = C.c_size_t(0)
+        nat.check(self.L.frb_decode_workspace_size(C.byref(p), total_frames, C.byref(ws_bytes)), "frb_decode_workspace_size")
+        return p, self._buf(ws_name, ws_bytes.value)
+
+    def _decode(self, launch, d_status: torch.Tensor, has_index: bool, allow_scan: bool, where: str) -> np.ndarray:
+        """Run decode_ladder over `launch(max_order, use_index)`, which enqueues one decode writing d_status.  When a decode
+        thread gave up waiting for a subframe offset, the engine switches to two-launch mode for good and runs the ladder once
+        more.  Every attempt ends in a synchronising status download, so the caller's staged tables are still alive then."""
+        def attempt(max_order, use_index):
+            launch(max_order, use_index)
+            return self._download(d_status, np.int32, 8).astype(np.int64)
+
+        status = decode_ladder(attempt, has_index, allow_scan, where)
+        if status[nat.ST_OFFSET_WAIT_TIMEOUTS] and not self._two_launch:
+            self._two_launch = True                  # offsets did not arrive inside the fused launch: separate skim launch from now on
+            status = decode_ladder(attempt, has_index, allow_scan, where)
+        return status
+
     def decode_streams(self, data: torch.Tensor, byte_offsets: np.ndarray, byte_lengths: np.ndarray, n_samples: np.ndarray,
                        sample_rates: np.ndarray, channels: int, bps: int, blocksize: int = 4096, verify_crc: bool = True,
                        sync: bool = True, name: str = "dec", index=None):
         """Frames of many streams (device bytes) -> int32 planar audio on the device.
 
-        data must be readable 16 bytes past the last stream.  Returns (audio, audio_base, status[8]).
-        sync=False leaves everything queued on the current stream and returns the status words as a device tensor
-        (the caller checks them, and status[4] != 0 means the stream needs the wide-order kernel: rerun with sync).
-        index = (frame_bytes, sub_bitoff) of these streams (EncodedTiles.index(), or the container's "frbI" blocks): the
-        sync scan and the subframe walk are skipped; an index that does not fit the streams is detected while decoding and
-        the call falls back to the scanning path."""
-        n_streams = len(n_samples)
-        n_samples = np.asarray(n_samples, dtype=np.int64)
-        frames_per = (n_samples + blocksize - 1) // blocksize
-        st = np.zeros(n_streams, dtype=nat.DECODE_STREAM_DTYPE)
-        st["byte_offset"] = byte_offsets
-        st["byte_length"] = byte_lengths
-        st["n_samples"] = n_samples
-        base = np.zeros(n_streams, dtype=np.int64)
-        np.cumsum(n_samples[:-1] * channels, out=base[1:])
-        st["audio_base"] = base
-        st["sample_rate"] = sample_rates
-        fb = np.zeros(n_streams, dtype=np.int64)
-        np.cumsum(frames_per[:-1], out=fb[1:])
-        st["frame_base"] = fb
-        total_frames = int(frames_per.sum())
-        total = int((n_samples * channels).sum())
+        data must be readable 16 bytes past the last stream.  Returns (audio, audio_base, status words).  sync=False makes
+        only the first attempt of decode_ladder, leaves it queued on the current stream and returns the status words as a
+        device tensor (the caller checks them: ST_LPC_ORDER_ABOVE_12 means rerun with sync).  index = (frame_bytes,
+        sub_bitoff) of these streams (EncodedTiles.index(), or the container's "frbI" blocks): the sync scan and the subframe
+        walk are skipped; an index that does not fit the streams is detected while decoding and the call scans instead."""
+        st, fstart = _stream_table(byte_offsets, byte_lengths, n_samples, sample_rates, channels, blocksize)
+        total_frames = int(fstart[-1])
+        base = st["audio_base"].copy()
         with torch.cuda.device(self.device):
             s = _stream_ptr()
-            audio = self._buf(name + "_audio", total * 4)
+            audio = self._buf(name + "_audio", int(st["n_samples"].sum()) * channels * 4)
             d_status = torch.zeros(8, dtype=torch.int32, device=self.device)
-            status = None
             idx = self._index_on_device(index, total_frames, channels)
-            for max_order, use_idx in ((12, True), (32, True), (12, False), (32, False)):
-                if use_idx and idx is None:
-                    continue
-                p = nat.DecodeParams(n_streams, channels, bps, blocksize, (1 if verify_crc else 0) | (2 if self._two_launch else 0), max_order)
-                ws_bytes = C.c_size_t(0)
-                nat.check(self.L.frb_decode_workspace_size(C.byref(p), total_frames, C.byref(ws_bytes)), "frb_decode_workspace_size")
-                ws = self._buf(name + "_ws", ws_bytes.value)
+
+            def launch(max_order, use_idx):
+                p, ws = self._decode_params(len(st), channels, bps, blocksize, verify_crc, max_order, total_frames, name + "_ws")
                 if use_idx:
                     nat.check(self.L.frb_decode_batch_indexed(C.byref(p), st.ctypes.data, data.data_ptr(), total_frames, idx[0].data_ptr(),
                                                               idx[1].data_ptr(), audio.data_ptr(), ws.data_ptr(), ws.numel(),
@@ -521,42 +583,25 @@ class Engine:
                 else:
                     nat.check(self.L.frb_decode_batch(C.byref(p), st.ctypes.data, data.data_ptr(), total_frames, audio.data_ptr(),
                                                       ws.data_ptr(), ws.numel(), d_status.data_ptr(), s), "frb_decode_batch")
-                if not sync:
-                    return audio, base, d_status
-                status = self._download(d_status, np.int32, 8).astype(np.int64)
-                if use_idx and (status[0] or status[1] or status[2]):
-                    idx = None                       # the index does not describe these bytes: decode again by scanning
-                    continue
-                if status[4] == 0:
-                    break
-        if status is not None and status[5] and not self._two_launch:
-            self._two_launch = True                  # offsets did not arrive inside the fused launch: separate skim launch from now on
-            return self.decode_streams(data, byte_offsets, byte_lengths, n_samples, sample_rates, channels, bps, blocksize, verify_crc,
-                                       sync, name, index)
+
+            if not sync:
+                launch(12, idx is not None)
+                return audio, base, d_status
+            status = self._decode(launch, d_status, idx is not None, True, "frb_decode_batch")
         return audio, base, status
 
     def _index_on_device(self, index, total_frames: int, channels: int):
-        """(frame_bytes, sub_bitoff) as int32 device tensors of the right length, or None."""
-        if index is None:
-            return None
-        fb, sb = index
-        if fb is None or (sb is None and channels > 1):
+        """(frame_bytes, sub_bitoff) as int32 device tensors, or None when they do not have the index's shape (_index_fits)."""
+        if not _index_fits(index, total_frames, channels):
             return None
 
-        def dev(x, n):
+        def dev(x):
             if isinstance(x, np.ndarray):
-                if x.size != n:
-                    return None
-                return self._upload(np.ascontiguousarray(x, dtype=np.uint32).view(np.uint8))[:4 * n].view(torch.int32)
-            if x.numel() != n:
-                return None
-            return x.contiguous() if x.is_cuda else self._upload(x.contiguous().numpy().view(np.uint8))[:4 * n].view(torch.int32)
+                return self._upload(np.ascontiguousarray(x, dtype=np.uint32).view(np.uint8))[:4 * x.size].view(torch.int32)
+            return x.contiguous() if x.is_cuda else self._upload(x.contiguous().numpy().view(np.uint8))[:4 * x.numel()].view(torch.int32)
 
-        d_fb = dev(fb, total_frames)
-        d_sb = dev(sb, total_frames * channels) if channels > 1 else d_fb
-        if d_fb is None or d_sb is None:
-            return None
-        return d_fb, d_sb
+        d_fb = dev(index[0])
+        return d_fb, dev(index[1]) if channels > 1 else d_fb
 
     def decode_tiles(self, data: torch.Tensor, byte_offsets: np.ndarray, byte_lengths: np.ndarray, tiles: np.ndarray,
                      sample_rates: np.ndarray, minmax: np.ndarray, scale: float, out: torch.Tensor, bps: int,
@@ -565,32 +610,19 @@ class Engine:
         denormalised in one launch (frb_decode_tiles); what `extract` + flac_to_tiff do per tile (cli.py:297-315,
         converter.py:181-253).  Returns the status words.  Two-band rasters go through decode_streams +
         denormalize_tiles (their frames may be mid/side coded); `fused` forces (True) or forbids (False) the one-launch
-        form, None picks it where it is the faster one."""
+        form, None picks it where it is the faster one (_fused_default)."""
         bands, H, W = out.shape
         n_tiles = len(tiles)
         n_samples = tiles["h"].astype(np.int64) * tiles["w"].astype(np.int64)
         _check_tile_sizes(n_samples)
         dt = str(out.dtype).replace("torch.", "")
-        # The fused launch pays off where the pixel mapping is the exact integer form (8/16-bit rasters behind 16-bit
-        # audio).  Wider dtypes need the fp64 formula per sample, which is cheaper in the bandwidth-bound mapping kernel
-        # than inside the issue-bound decode kernel (C4 float32: 129 vs 97 GSamples/s), so they stay two-step.
-        if fused is None:
-            fused = bps == 16 and dt in ("uint8", "int8", "uint16", "int16") and float(scale) == 32767.0
-        if bands == 2 or not fused:
+        if bands == 2 or not (_fused_default(bps, dt, scale) if fused is None else fused):
             audio, base, status = self.decode_streams(data, byte_offsets, byte_lengths, n_samples, sample_rates, bands, bps, blocksize,
                                                       verify_crc, index=index)
             self.denormalize_tiles(audio, base, tiles, minmax, scale, out)
             return status
-        frames_per = (n_samples + blocksize - 1) // blocksize
-        st = np.zeros(n_tiles, dtype=nat.DECODE_STREAM_DTYPE)
-        st["byte_offset"] = byte_offsets
-        st["byte_length"] = byte_lengths
-        st["n_samples"] = n_samples
-        st["sample_rate"] = sample_rates
-        fb = np.zeros(n_tiles, dtype=np.int64)
-        np.cumsum(frames_per[:-1], out=fb[1:])
-        st["frame_base"] = fb
-        total_frames = int(frames_per.sum())
+        st, fstart = _stream_table(byte_offsets, byte_lengths, n_samples, sample_rates, bands, blocksize)
+        total_frames = int(fstart[-1])
         with torch.cuda.device(self.device):
             s = _stream_ptr()
             # one staging buffer, one copy: tile table followed by the min/max pairs
@@ -599,15 +631,10 @@ class Engine:
             stage[n_tiles * 16:] = np.ascontiguousarray(minmax, dtype=np.float64).reshape(-1).view(np.uint8)
             d_stage = self._upload(stage)
             d_status = torch.zeros(8, dtype=torch.int32, device=self.device)
-            status = None
             idx = self._index_on_device(index, total_frames, bands)
-            for max_order, use_idx in ((12, True), (32, True), (12, False), (32, False)):
-                if use_idx and idx is None:
-                    continue
-                p = nat.DecodeParams(n_tiles, bands, bps, blocksize, (1 if verify_crc else 0) | (2 if self._two_launch else 0), max_order)
-                ws_bytes = C.c_size_t(0)
-                nat.check(self.L.frb_decode_workspace_size(C.byref(p), total_frames, C.byref(ws_bytes)), "frb_decode_workspace_size")
-                ws = self._buf("dec_ws", ws_bytes.value)
+
+            def launch(max_order, use_idx):
+                p, ws = self._decode_params(n_tiles, bands, bps, blocksize, verify_crc, max_order, total_frames, "dec_ws")
                 if use_idx:
                     nat.check(self.L.frb_decode_tiles_indexed(C.byref(p), st.ctypes.data, data.data_ptr(), total_frames,
                                                               idx[0].data_ptr(), idx[1].data_ptr(),
@@ -619,20 +646,8 @@ class Engine:
                                                       d_stage.data_ptr(), d_stage.data_ptr() + n_tiles * 16, float(scale),
                                                       out.data_ptr(), nat.DTYPE_CODES[dt], bands, H, W,
                                                       ws.data_ptr(), ws.numel(), d_status.data_ptr(), s), "frb_decode_tiles")
-                status = self._download(d_status, np.int32, 8).astype(np.int64)      # (synchronises: d_stage stays alive until the kernels are done)
-                if status[6]:
-                    raise nat.NativeError(nat.ERR_INVALID_ARG, "frb_decode_tiles",
-                                          f"{int(status[6])} tile(s) do not match their stream length or lie outside the raster")
-                if use_idx and (status[0] or status[1] or status[2]):
-                    idx = None                       # the index does not describe these bytes: decode again by scanning
-                    continue
-                if status[4] == 0:
-                    break
-        if status[5] and not self._two_launch:
-            self._two_launch = True                  # offsets did not arrive inside the fused launch: separate skim launch from now on
-            return self.decode_tiles(data, byte_offsets, byte_lengths, tiles, sample_rates, minmax, scale, out, bps, blocksize, verify_crc,
-                                     fused, index)
-        return status
+
+            return self._decode(launch, d_status, idx is not None, True, "frb_decode_tiles")
 
     def decode_window(self, data: torch.Tensor, byte_offsets: np.ndarray, byte_lengths: np.ndarray, tiles: np.ndarray,
                       sample_rates: np.ndarray, minmax: np.ndarray, scale: float, window, out: torch.Tensor, bps: int,
@@ -640,7 +655,7 @@ class Engine:
                       fused: Optional[bool] = None) -> np.ndarray:
         """The pixels of `window` (col_off, row_off, width, height, image coordinates) from the frames of the tiles that
         cover it (image coordinates) -> the (bands, height, width) device array `out`.  Only the frames each tile's part of
-        the window needs are decoded (window_frames).  Returns the status words; status[3] counts the decoded frames.
+        the window needs are decoded (window_frames).  Returns the status words; ST_FRAMES_DECODED counts the decoded frames.
         byte_offsets / byte_lengths: where each tile's frames are in `data` -- all of them, or with `runs_only` only the
         run's frames (a partial read; then the seek index is required, and a rejected index is reported in the status words
         instead of falling back to a scan, which would need every frame).  index: (frame_bytes, sub_bitoff) of all the
@@ -651,15 +666,10 @@ class Engine:
             raise ValueError("out must have the window's shape")
         n_samples = tiles["h"].astype(np.int64) * tiles["w"].astype(np.int64)
         _check_tile_sizes(n_samples)
-        frames_all = (n_samples + blocksize - 1) // blocksize
-        fstart = np.concatenate([[0], np.cumsum(frames_all)])
-        if index is not None and index[0] is not None and (bands == 1 or index[1] is not None):
-            fb_all = np.asarray(index[0]).view(np.uint32).reshape(-1)
-            sb_all = np.asarray(index[1]).view(np.uint32).reshape(-1) if bands > 1 else None
-            if fb_all.size != fstart[-1] or (sb_all is not None and sb_all.size != fstart[-1] * bands):
-                fb_all = sb_all = None
-        else:
-            fb_all = sb_all = None
+        fstart = _stream_table(byte_offsets, byte_lengths, n_samples, sample_rates, bands, blocksize)[1]
+        fits = _index_fits(index, int(fstart[-1]), bands)
+        fb_all = np.asarray(index[0]).view(np.uint32).reshape(-1) if fits else None
+        sb_all = np.asarray(index[1]).view(np.uint32).reshape(-1) if fits and bands > 1 else None
         if runs_only and fb_all is None:
             raise ValueError("decode_window(runs_only=True) needs the tiles' seek index")
         runs = window_frames(tiles, window, blocksize,
@@ -669,21 +679,15 @@ class Engine:
         sel = runs["tile"]
         n_runs = len(runs)
         dt = str(out.dtype).replace("torch.", "")
-        if fused is None:          # the rule decode_tiles measured: the exact integer form fused, the fp64 formula two-step
-            fused = bps == 16 and dt in ("uint8", "int8", "uint16", "int16") and float(scale) == 32767.0
-        two_step = bands == 2 or not fused
+        two_step = bands == 2 or not (_fused_default(bps, dt, scale) if fused is None else fused)
         run_n = np.minimum((runs["first_frame"] + runs["n_frames"]) * blocksize, n_samples[sel]) - runs["first_frame"] * blocksize
         st = np.zeros(n_runs, dtype=nat.WINDOW_STREAM_DTYPE)
         st["total_samples"] = n_samples[sel]
         st["sample_rate"] = np.asarray(sample_rates)[sel]
         st["first_frame"] = runs["first_frame"]
         st["n_frames"] = runs["n_frames"]
-        fbase = np.zeros(n_runs, dtype=np.int64)
-        np.cumsum(runs["n_frames"][:-1], out=fbase[1:])
-        st["frame_base"] = fbase
-        abase = np.zeros(n_runs, dtype=np.int64)
-        np.cumsum(run_n[:-1] * bands, out=abase[1:])
-        st["audio_base"] = abase
+        st["frame_base"][1:] = np.cumsum(runs["n_frames"][:-1])
+        st["audio_base"][1:] = np.cumsum(run_n[:-1] * bands)
         total_frames = int(runs["n_frames"].sum())
         idx_host = None
         if fb_all is not None:
@@ -703,40 +707,23 @@ class Engine:
             idx = None if idx_host is None else self._index_on_device(idx_host, total_frames, bands)
             audio = self._buf("win_audio", int(run_n.sum()) * bands * 4) if two_step else None
             win = nat.Tile(row0, col0, height, width)
-            status = None
-            for max_order, use_idx in ((12, True), (32, True), (12, False), (32, False)):
-                if use_idx and idx is None:
-                    continue
-                if not use_idx and runs_only:
-                    break                            # the scan path needs every frame of the streams: the caller decides
+
+            def launch(max_order, use_idx):
                 if use_idx:
                     st["byte_offset"] = offs if runs_only else offs + runs["byte_offset"]
                     st["byte_length"] = lens if runs_only else runs["byte_length"]
                 else:
                     st["byte_offset"], st["byte_length"] = offs, lens
-                p = nat.DecodeParams(n_runs, bands, bps, blocksize, (1 if verify_crc else 0) | (2 if self._two_launch else 0), max_order)
-                ws_bytes = C.c_size_t(0)
-                nat.check(self.L.frb_decode_workspace_size(C.byref(p), total_frames, C.byref(ws_bytes)), "frb_decode_workspace_size")
-                ws = self._buf("dec_ws", ws_bytes.value)
+                p, ws = self._decode_params(n_runs, bands, bps, blocksize, verify_crc, max_order, total_frames, "dec_ws")
                 nat.check(self.L.frb_decode_window(C.byref(p), st.ctypes.data, data.data_ptr(), total_frames,
                                                    idx[0].data_ptr() if use_idx else None, idx[1].data_ptr() if use_idx else None,
                                                    d_stage.data_ptr(), d_stage.data_ptr() + n_runs * 16, float(scale), win,
                                                    audio.data_ptr() if two_step else out.data_ptr(), -1 if two_step else nat.DTYPE_CODES[dt],
                                                    ws.data_ptr(), ws.numel(), d_status.data_ptr(), s), "frb_decode_window")
-                status = self._download(d_status, np.int32, 8).astype(np.int64)      # (synchronises: d_stage stays alive)
-                if status[6]:
-                    raise nat.NativeError(nat.ERR_INVALID_ARG, "frb_decode_window",
-                                          f"{int(status[6])} tile(s) do not hold as many pixels as their stream has samples")
-                if use_idx and (status[0] or status[1] or status[2]):
-                    idx = None                       # the index does not describe these bytes: decode again by scanning
-                    continue
-                if status[4] == 0:
-                    break
-            if status[5] and not self._two_launch:
-                self._two_launch = True              # offsets did not arrive inside the fused launch: separate skim launch from now on
-                return self.decode_window(data, byte_offsets, byte_lengths, tiles, sample_rates, minmax, scale, window, out, bps,
-                                          blocksize, index, runs_only, verify_crc, fused)
-            if two_step and not (status[0] or status[1] or status[2] or status[4] or status[5]):
+
+            # the scan path needs every frame of the streams: with runs_only the caller decides what a rejected index means
+            status = self._decode(launch, d_status, idx is not None, not runs_only, "frb_decode_window")
+            if two_step and not (nat.status_damaged(status) or status[nat.ST_LPC_ORDER_ABOVE_12] or status[nat.ST_OFFSET_WAIT_TIMEOUTS]):
                 d_st = self._upload(st)
                 nat.check(self.L.frb_denormalize_window(audio.data_ptr(), d_st.data_ptr(), n_runs, blocksize, d_stage.data_ptr(),
                                                         d_stage.data_ptr() + n_runs * 16, float(scale), win, out.data_ptr(),
@@ -760,8 +747,8 @@ class Engine:
         byte_offsets = np.asarray(byte_offsets, dtype=np.int64)
         byte_lengths = np.asarray(byte_lengths, dtype=np.int64)
         # seek index: uploaded once, sliced per stage by frame range (tiles and frames are in payload order)
-        frames_per = (tiles["h"].astype(np.int64) * tiles["w"].astype(np.int64) + blocksize - 1) // blocksize
-        frame_start = np.concatenate([[0], np.cumsum(frames_per)])
+        frame_start = _stream_table(byte_offsets, byte_lengths, tiles["h"].astype(np.int64) * tiles["w"].astype(np.int64), sample_rates,
+                                    bands, blocksize)[1]
         with torch.cuda.device(self.device):
             d_index = self._index_on_device(index, int(frame_start[-1]), bands)
         spans = [(int(byte_offsets[i0]), int(byte_offsets[i1 - 1] + byte_lengths[i1 - 1])) for i0, i1, _, _ in groups]

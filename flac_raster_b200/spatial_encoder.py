@@ -780,7 +780,7 @@ class SpatialFLACStreamer:
             "dtype": str(dtype), "nodata": md0.get("nodata"), "transform": affine9(wt) if tr else None,
             "bounds": {"left": left, "bottom": top + height * wt[4], "right": left + width * wt[0], "top": top},
             "window": {"col_off": col0, "row_off": row0, "width": width, "height": height},
-            "tiles": [f.frame_id for f in sel], "frames_decoded": int(status[3]),
+            "tiles": [f.frame_id for f in sel], "frames_decoded": int(status[nat.ST_FRAMES_DECODED]),
         }
         return out.cpu().numpy(), meta
 
