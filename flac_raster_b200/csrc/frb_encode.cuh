@@ -1473,21 +1473,35 @@ extern "C" int frb_encode_analyse(const frb_encode_params *p, const void *d_audi
         const bool wide = p->bps > 16;
         // one CTA per subframe; with mid/side the 17-bit side channel (virtual channel 3) runs in the 64-bit kernels
         const dim3 grid((uint32_t)frames, ms ? 3u : p->channels), grid_side((uint32_t)frames, 1);
+        // 16-bit subframes: one warp each, FIXED search included (k_enc_stats_warp); FRB_STATS_CTA=1 selects the CTA kernel
+        // and k_enc_fixed for them as well (A/B runs).  The 32-bps and side-channel subframes always take the CTA kernel.
+        static int stats_cta = -1;
+        if (stats_cta < 0) { const char *e = getenv("FRB_STATS_CTA"); stats_cta = e ? atoi(e) : 0; }
+        const bool warp_stats = !wide && stats_cta != 1;
+        const uint32_t main_ch = ms ? 3u : p->channels;
         prof_begin(4, s);
 #define FRB_STATS(W, NL, G, C0, EX) k_enc_stats<W, NL><<<G, kEncThreads, 0, s>>>(w.frame_table, an_ch, p->bps, windows, (uint32_t)cfg.max_po, an_audio, \
             w.window, w.stats, w.autoc, w.fx_fin, C0, EX)
-#define FRB_STATS_L(NL) do { if (wide) FRB_STATS(true, NL, grid, 0u, 0u); else FRB_STATS(false, NL, grid, 0u, 0u); \
+#define FRB_STATS_WARP(NL) k_enc_stats_warp<NL><<<(uint32_t)((frames * main_ch + kStatsWarps - 1) / kStatsWarps), kStatsWarps * 32, 0, s>>>( \
+            w.frame_table, an_ch, main_ch, (uint32_t)(frames * main_ch), p->bps, windows, (uint32_t)cfg.max_po, an_audio, w.window, w.stats, w.autoc)
+#define FRB_STATS_L(NL) do { if (warp_stats) FRB_STATS_WARP(NL); else if (wide) FRB_STATS(true, NL, grid, 0u, 0u); else FRB_STATS(false, NL, grid, 0u, 0u); \
                              if (ms) FRB_STATS(true, NL, grid_side, 3u, 1u); } while (0)
         if (max_lpc == 0) FRB_STATS_L(0);
         else if (max_lpc <= 8) FRB_STATS_L(9);
         else FRB_STATS_L(13);
 #undef FRB_STATS_L
+#undef FRB_STATS_WARP
 #undef FRB_STATS
-        prof_end(4, s);
         FRB_LAUNCH_CHECK("k_enc_stats");
-        k_enc_fixed<<<(total_tasks + 3) / 4, 128, 0, s>>>(w.frame_table, an_ch, p->bps, (uint32_t)cfg.max_po, total_tasks, an_audio,
-                                                        w.stats, w.fx_fin, side_ch);
-        FRB_LAUNCH_CHECK("k_enc_fixed");
+        // the FIXED search of the subframes k_enc_stats analysed: all of them, or only the side channel
+        const uint32_t fx_c0 = warp_stats ? 3u : 0u, fx_nch = warp_stats ? 1u : an_ch;
+        if (!warp_stats || ms) {
+            const uint32_t fx_total = (uint32_t)(frames * fx_nch);
+            k_enc_fixed<<<(fx_total + 3) / 4, 128, 0, s>>>(w.frame_table, an_ch, fx_c0, fx_nch, p->bps, (uint32_t)cfg.max_po, fx_total,
+                                                         an_audio, w.stats, w.fx_fin, side_ch);
+            FRB_LAUNCH_CHECK("k_enc_fixed");
+        }
+        prof_end(4, s);
         const uint32_t n_slots = n_cands;
         const uint32_t model_threads = total_tasks * n_slots;
         if (n_cands) {

@@ -7,10 +7,13 @@
 // 64-bit shuffles, and 255 of 256 threads idled at a barrier while lane 0 ran Levinson-Durbin, the order
 // estimate (logarithms) and the coefficient quantisation in fp64.  Here the work is split where the data
 // dependencies are:
-//   k_enc_stats   CTA per subframe, 16 samples per thread held in REGISTERS (+12 halo samples read
-//                 straight from global/L1): wasted bits, constant check, fixed-predictor abs sums
-//                 (32-bit, REDUX warp sums), windowed autocorrelation for every apodization of the
-//                 level (fp64 FMA chain in registers) -> ~200 bytes of statistics per subframe
+//   k_enc_stats_warp  WARP per 16-bit subframe, 4 subframes per 128-thread CTA, no barrier: lane l walks the
+//                 16-sample chunks 32j + l (j = 0..7) in registers (+12 halo samples read straight from
+//                 global/L1): wasted bits, constant check, fixed-predictor abs sums (32-bit, REDUX warp
+//                 sums), windowed autocorrelation for every apodization of the level (fp64 FMA chain in
+//                 registers), and the FIXED candidate's Rice search -> ~200 bytes of statistics per subframe
+//   k_enc_stats   the same per CTA (16 samples per thread) for the 32-bps and side-channel subframes (and
+//                 every subframe with FRB_STATS_CTA=1); k_enc_fixed then runs their FIXED search
 //   k_enc_model   ONE THREAD per (subframe, apodization): Levinson-Durbin, libFLAC's order estimate
 //                 and coefficient quantisation -- the serial fp64 section now runs 32 subframes per
 //                 warp instead of one lane per CTA -> candidate predictors (64 bytes each)
@@ -20,11 +23,12 @@
 //                 128-bit slot copy
 // All decisions are the same as the one-kernel encoder's (and the oracle's): same estimates, same
 // tie-breaks, same fp64 operation order in the model; the autocorrelation uses the same per-thread /
-// butterfly / cross-warp summation tree as before.
+// butterfly / cross-warp summation tree as before (in k_enc_stats_warp: per chunk / butterfly / running sum
+// over the chunk rows, the same additions).
 #pragma once
 
 constexpr int kMaxSets = 6;        // autocorrelation sets per subframe: root, 2 halves, 3 thirds (level 8)
-constexpr int kMaxCands = 9;       // LPC candidates per subframe (level 8: 1 + 2 + 6); the FIXED candidate is searched in k_enc_stats
+constexpr int kMaxCands = 9;       // LPC candidates per subframe (level 8: 1 + 2 + 6); the FIXED candidate is searched before k_enc_code
 constexpr int kLags = kMaxOrd + 1;
 
 struct EncSubStats {
@@ -277,6 +281,101 @@ __device__ __forceinline__ void warp_search(const unsigned long long *fin, uint3
     *rb_out = rb; *best_l_out = best_l;
 }
 
+// ------------------------------------------------------------------------------------------------ autocorrelation
+// One chunk = the 16 samples [16t, 16t + 16) of a block (k_enc_stats' thread t), at xs[12..27] with the 12 samples before
+// them at xs[0..11] (zeros for t = 0).  Both statistics kernels form the windowed autocorrelation of a chunk with these
+// helpers, so their fp64 partials are the same bits.
+
+// full-length window for the chunk's samples and its HALO samples
+template <int HALO>
+__device__ __forceinline__ void load_window_chunk(const float *__restrict__ window, int t, float (&wv)[kSPT + HALO + 1]) {
+    const float4 *wp = reinterpret_cast<const float4 *>(window + t * kSPT) - HALO / 4;
+#pragma unroll
+    for (int q = 0; q < (kSPT + HALO) / 4; q++) {
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (t > 0 || q >= HALO / 4) v = __ldg(wp + q);
+        wv[4 * q] = v.x; wv[4 * q + 1] = v.y; wv[4 * q + 2] = v.z; wv[4 * q + 3] = v.w;
+    }
+}
+
+// windowed samples (libFLAC windows in single precision): the full window (set 0) ...
+template <int HALO>
+__device__ __forceinline__ void window_full(const int32_t (&xs)[28], const float (&wv)[kSPT + HALO + 1], float (&df)[kSPT + HALO]) {
+    // chunk 0's halo samples are zero, so no range checks are needed
+#pragma unroll
+    for (int j = 0; j < kSPT + HALO; j++) df[j] = __fmul_rn((float)xs[12 - HALO + j], wv[j]);
+}
+// ... and a subdivide_tukey part: window[0, part) and its last `part` values around a flat top, over [wshift, wshift + wlen)
+template <int HALO>
+__device__ __forceinline__ void window_part(const int32_t (&xs)[28], uint32_t i0, uint32_t wshift, uint32_t wlen, uint32_t part,
+                                            const float *__restrict__ window, float (&df)[kSPT + HALO]) {
+    constexpr uint32_t n = kMaxBlock;
+#pragma unroll
+    for (int j = 0; j < kSPT + HALO; j++) {
+        const int idx = (int)i0 - HALO + j;
+        float v = 0.0f;
+        if (idx >= (int)wshift && (uint32_t)idx < wshift + wlen) {
+            const uint32_t local = (uint32_t)idx - wshift;
+            float w1;
+            if (local < part) w1 = __ldg(window + local);
+            else if (local < 2 * part) w1 = __ldg(window + (n - 2 * part + local));
+            else w1 = 0.0f;
+            v = __fmul_rn((float)xs[12 - HALO + j], w1);
+        }
+        df[j] = v;
+    }
+}
+
+// the chunk's partial autocorrelation: sliding window of the last NLAGS samples in double (one conversion per sample, few
+// live registers), one FMA chain per lag from ac[] (the callers start it at 0.0)
+template <int NLAGS>
+__device__ __forceinline__ void autoc_fma(const float (&df)[kSPT + NLAGS - 1], double (&ac)[NLAGS]) {
+    constexpr int HALO = NLAGS - 1;
+    double win[NLAGS];
+#pragma unroll
+    for (int l = 1; l < NLAGS; l++) win[l] = (double)df[HALO - l];
+#pragma unroll
+    for (int s = 0; s < kSPT; s++) {
+        if (s > 0) {
+#pragma unroll
+            for (int l = NLAGS - 1; l >= 1; l--) win[l] = win[l - 1];
+        }
+        win[0] = (double)df[HALO + s];
+#pragma unroll
+        for (int l = 0; l < NLAGS; l++) ac[l] = fma(win[0], win[l], ac[l]);
+    }
+}
+
+// Warp totals of the 32 lanes' partials (same pairing tree as an xor butterfly per lag): lags 0-7 split over the lanes (lag
+// autoc_lag8(lane) in g8, complete in the lanes with lane % 4 == 0), lag 8 in every lane (g1), lags 9-12 when NLAGS == 13
+// (lag autoc_lag4(lane) in g4, complete in the lanes with lane % 8 == 0).
+__device__ __forceinline__ int autoc_lag8(int lane) { return ((lane >> 4) & 1) * 4 + ((lane >> 3) & 1) * 2 + ((lane >> 2) & 1); }
+__device__ __forceinline__ int autoc_lag4(int lane) { return 9 + ((lane >> 4) & 1) * 2 + ((lane >> 3) & 1); }
+template <int NLAGS>
+__device__ __forceinline__ void autoc_warp_sums(const double (&ac)[NLAGS], int lane, double &g8, double &g1, double &g4) {
+    double v8[8];
+#pragma unroll
+    for (int l = 0; l < 8; l++) v8[l] = ac[l];
+    warp_sum_split<8>(v8, lane);
+    double v1[1] = {ac[8]};
+    warp_sum_split<1>(v1, lane);
+    g8 = v8[0]; g1 = v1[0]; g4 = 0.0;
+    if constexpr (NLAGS > 9) {
+        double v4[4];
+#pragma unroll
+        for (int l = 0; l < 4; l++) v4[l] = ac[9 + l];
+        warp_sum_split<4>(v4, lane);
+        g4 = v4[0];
+    }
+}
+
+// libFLAC's "bits per sample" estimate of the guessed FIXED order (FLAC__fixed_compute_best_predictor); the FIXED candidate
+// is not tried when it reaches the subframe's bps
+__device__ __forceinline__ float fixed_bits_estimate(unsigned long long eg) {
+    constexpr uint32_t n = kMaxBlock;
+    return (float)(eg > 0 ? log(0.69314718055994530942 * (double)eg / (double)(n - 4)) / 0.69314718055994530942 : 0.0);
+}
+
 // ------------------------------------------------------------------------------------------------ stats
 struct StatsShared {
     uint32_t orv[8], diff[8];
@@ -320,15 +419,7 @@ k_enc_stats(const FrameDesc *__restrict__ frames, uint32_t channels, uint32_t bp
     // full-length window for this thread's samples and halo
     float wv[kSPT + HALO + 1];
     auto load_window = [&]() {
-        if (NLAGS > 0) {
-            const float4 *wp = reinterpret_cast<const float4 *>(window + tid * kSPT) - HALO / 4;
-#pragma unroll
-            for (int q = 0; q < (kSPT + HALO) / 4; q++) {
-                float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (tid > 0 || q >= HALO / 4) v = __ldg(wp + q);
-                wv[4 * q] = v.x; wv[4 * q + 1] = v.y; wv[4 * q + 2] = v.z; wv[4 * q + 3] = v.w;
-            }
-        }
+        if constexpr (NLAGS > 0) load_window_chunk<HALO>(window, tid, wv);
     };
 #if !FRB_STATS_LATEWIN
     load_window();          // fetched together with the samples
@@ -445,7 +536,8 @@ k_enc_stats(const FrameDesc *__restrict__ frames, uint32_t channels, uint32_t bp
         flags |= 2u;
     }
     if (tid == 5) { stats[task].wasted = wasted; stats[task].flags = flags; }
-    if (NLAGS == 0 || diff == 0) return;
+    if (diff == 0) return;
+    if constexpr (NLAGS > 0) {
     // ---- windowed autocorrelation, one set per apodization (root, halves, thirds) ----
 #if FRB_STATS_LATEWIN
     // the window (16 KB, shared by every CTA: L1 hits) and, with FRB_STATS_RELOAD, the samples are fetched only now: the
@@ -460,12 +552,12 @@ k_enc_stats(const FrameDesc *__restrict__ frames, uint32_t channels, uint32_t bp
         for (uint32_t sub = 0; sub < nsub; sub++, set++) {
             uint32_t wshift = 0, wlen = n, part = 0;
             if (b > 1) { part = n / b / 2; wshift = (sub * n) / b; wlen = n / b; }
-            double ac[NLAGS > 0 ? NLAGS : 1];
+            double ac[NLAGS];
 #pragma unroll
             for (int l = 0; l < NLAGS; l++) ac[l] = 0.0;
             // threads whose 16 samples lie outside the window contribute nothing
             if (i0 + kSPT > wshift && i0 < wshift + wlen) {
-                float df[kSPT + HALO];                   // windowed samples (libFLAC windows in single precision)
+                float df[kSPT + HALO];
                 // 16-bit kernels at the 64-register cap: the samples are fetched again per window set (L1 hits) so that they
                 // are dead once df[] is formed, instead of staying in 28 registers next to the fp64 window and accumulators
                 // for the next set.  (The 64-bit / 13-lag instantiations run at 128 registers and keep them: reloading
@@ -480,60 +572,16 @@ k_enc_stats(const FrameDesc *__restrict__ frames, uint32_t channels, uint32_t bp
                     }
                 }
                 const int32_t (&xs)[28] = pick_ref<RELOAD>(xr, xs0);
-                if (b == 1) {
-                    // full window: thread 0's halo samples are zero, so no range checks are needed
-#pragma unroll
-                    for (int j = 0; j < kSPT + HALO; j++) df[j] = __fmul_rn((float)xs[12 - HALO + j], wv[j]);
-                } else {
-#pragma unroll
-                    for (int j = 0; j < kSPT + HALO; j++) {
-                        const int idx = (int)i0 - HALO + j;
-                        float v = 0.0f;
-                        if (idx >= (int)wshift && (uint32_t)idx < wshift + wlen) {
-                            const uint32_t local = (uint32_t)idx - wshift;
-                            float w1;
-                            if (local < part) w1 = __ldg(window + local);
-                            else if (local < 2 * part) w1 = __ldg(window + (n - 2 * part + local));
-                            else w1 = 0.0f;
-                            v = __fmul_rn((float)xs[12 - HALO + j], w1);
-                        }
-                        df[j] = v;
-                    }
-                }
-                // sliding window of the last NLAGS samples in double: one conversion per sample, few live registers
-                double win[NLAGS > 0 ? NLAGS : 1];
-#pragma unroll
-                for (int l = 1; l < NLAGS; l++) win[l] = (double)df[HALO - l];
-#pragma unroll
-                for (int s = 0; s < kSPT; s++) {
-                    if (s > 0) {
-#pragma unroll
-                        for (int l = NLAGS - 1; l >= 1; l--) win[l] = win[l - 1];
-                    }
-                    win[0] = (double)df[HALO + s];
-#pragma unroll
-                    for (int l = 0; l < NLAGS; l++) ac[l] = fma(win[0], win[l], ac[l]);
-                }
+                if (b == 1) window_full<HALO>(xs, wv, df);
+                else window_part<HALO>(xs, i0, wshift, wlen, part, window, df);
+                autoc_fma<NLAGS>(df, ac);
             }
-            // warp sums (same pairing tree as an xor butterfly per lag), lags 0-7 split over the lanes
-            {
-                double g8[8];
-#pragma unroll
-                for (int l = 0; l < 8; l++) g8[l] = ac[l];
-                warp_sum_split<8>(g8, lane);
-                double g1[1] = {ac[8]};
-                warp_sum_split<1>(g1, lane);
-                __syncthreads();                          // previous set's S.ac has been consumed
-                if ((lane & 3) == 0) S.ac[warp][((lane >> 4) & 1) * 4 + ((lane >> 3) & 1) * 2 + ((lane >> 2) & 1)] = g8[0];
-                if (lane == 0) S.ac[warp][8] = g1[0];
-                if (NLAGS > 9) {
-                    double g4[4];
-#pragma unroll
-                    for (int l = 0; l < 4; l++) g4[l] = ac[(NLAGS > 9 ? 9 : 0) + l];
-                    warp_sum_split<4>(g4, lane);
-                    if ((lane & 7) == 0) S.ac[warp][9 + ((lane >> 4) & 1) * 2 + ((lane >> 3) & 1)] = g4[0];
-                }
-            }
+            double g8, g1, g4;
+            autoc_warp_sums<NLAGS>(ac, lane, g8, g1, g4);
+            __syncthreads();                          // previous set's S.ac has been consumed
+            if ((lane & 3) == 0) S.ac[warp][autoc_lag8(lane)] = g8;
+            if (lane == 0) S.ac[warp][8] = g1;
+            if (NLAGS > 9 && (lane & 7) == 0) S.ac[warp][autoc_lag4(lane)] = g4;
             __syncthreads();
             if (tid < NLAGS) {
                 double s = 0.0;
@@ -543,31 +591,31 @@ k_enc_stats(const FrameDesc *__restrict__ frames, uint32_t channels, uint32_t bp
             }
         }
     }
+    }
 }
 
 // ------------------------------------------------------------------------------------------------ fixed search
 // One warp per subframe: libFLAC's "is FIXED worth trying" estimate and the Rice search of the FIXED candidate
-// from the finest partition sums k_enc_stats stored.
+// from the finest partition sums k_enc_stats stored.  Runs over channels [c0, c0 + nch) of every frame (the subframes
+// k_enc_stats analysed; k_enc_stats_warp searches its own).
 __global__ void __launch_bounds__(128)
-k_enc_fixed(const FrameDesc *__restrict__ frames, uint32_t channels, uint32_t bps_stream, uint32_t max_po_cfg, uint32_t total_tasks,
-            const EncSrc audio, EncSubStats *__restrict__ stats, const unsigned long long *__restrict__ fx_fin,
+k_enc_fixed(const FrameDesc *__restrict__ frames, uint32_t channels, uint32_t c0, uint32_t nch, uint32_t bps_stream, uint32_t max_po_cfg,
+            uint32_t total, const EncSrc audio, EncSubStats *__restrict__ stats, const unsigned long long *__restrict__ fx_fin,
             uint32_t side_ch) {
     const int lane = threadIdx.x & 31;
-    const uint32_t task = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (task >= total_tasks) return;
-    const uint32_t f = task / channels;
-    const TaskLoc L = locate_task(frames, audio, f, task - f * channels);
+    const uint32_t g = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (g >= total) return;
+    const uint32_t f = g / nch, ch = c0 + (g - f * nch), task = f * channels + ch;
+    const TaskLoc L = locate_task(frames, audio, f, ch);
     if (!fast_eligible(L)) return;
     EncSubStats *st = stats + task;
     const uint32_t flags = st->flags;
     if (!(flags & 2u)) return;
-    constexpr uint32_t n = kMaxBlock;
     const uint32_t wasted = st->wasted, guess = st->fx_order;
-    const uint32_t bps = bps_stream + (task - f * channels == side_ch ? 1u : 0u) - wasted;
+    const uint32_t bps = bps_stream + (ch == side_ch ? 1u : 0u) - wasted;
     // FLAC__fixed_compute_best_predictor's estimate for the guessed order; >= bps means "do not even try"
     const unsigned long long eg = st->e[guess];
-    const float fbits_guess = (float)(eg > 0 ? log(0.69314718055994530942 * (double)eg / (double)(n - 4)) / 0.69314718055994530942 : 0.0);
-    if (fbits_guess >= (float)bps || st->fx_bad) {
+    if (fixed_bits_estimate(eg) >= (float)bps || st->fx_bad) {
         __syncwarp();
         if (lane == 0) st->flags = flags & ~2u;
         return;
@@ -575,6 +623,193 @@ k_enc_fixed(const FrameDesc *__restrict__ frames, uint32_t channels, uint32_t bp
     uint32_t rb, best_l;
     warp_search(fx_fin + (size_t)task * 64, guess, max_po_cfg, bps_stream > 16 ? 31u : 15u, lane, st->fx_params, &rb, &best_l);
     if (lane == 0) { st->fx_bits = 8 + wasted + guess * bps + rb; st->fx_po = max_po_cfg - best_l; }
+}
+
+// ------------------------------------------------------------------------------------------------ stats, warp per subframe
+// k_enc_stats and k_enc_fixed for a 16-bit subframe (!WIDE) in ONE warp, with no CTA barrier: lane l walks chunks j = 0..7,
+// chunk (j, l) being the 16 samples of k_enc_stats' thread t = 32j + l, with the same halo and window values, so every
+// partial sum is the one that thread formed.
+//  * one pass over the samples gives the OR / XOR for wasted bits and constant, the fixed-predictor sums and the root
+//    window's autocorrelation, all from the UNSHIFTED samples; the wasted-bits shift is applied afterwards, exactly:
+//    every sample is a multiple of 2^w, so a |residual| sum shifts right by w without remainder, and in the window product,
+//    the fp64 FMA chain and the sums every value scales by a power of two with no rounding change (no value comes near
+//    the subnormal range), so the root set times 2^-2w is the same bits as k_enc_stats' result from shifted samples;
+//  * the per-chunk warp totals of the autocorrelation (warp_sum_split, as k_enc_stats) go into a running total per lag in
+//    chunk order from 0.0: k_enc_stats' cross-warp sum over its 8 warps, the same additions in the same order;
+//  * the five per-chunk |residual| sums go to shared memory, so the guessed order's finest partition sums (64..512
+//    samples = 4..32 chunks) need no second pass, and the FIXED candidate's Rice search (warp_search) runs here.
+// The subdivide_tukey sets (levels 6-8) take one more pass each over the chunk rows they overlap, from shifted samples.
+struct StatsWarpShared {
+    uint32_t ch[5][kEncThreads];            // |order-q residual| sum of chunk t = 32j + lane (unshifted samples)
+    unsigned long long fin[64];             // finest partition sums of the guessed order
+};
+constexpr int kStatsWarps = 4;              // warps (subframes) per CTA
+
+#ifndef FRB_STATS_WARP_MINB
+#define FRB_STATS_WARP_MINB 6
+#endif
+template <int NLAGS>
+__global__ void __launch_bounds__(kStatsWarps * 32, FRB_STATS_WARP_MINB)
+k_enc_stats_warp(const FrameDesc *__restrict__ frames, uint32_t channels, uint32_t nch, uint32_t total, uint32_t bps_stream,
+                 uint32_t windows, uint32_t max_po_cfg, const EncSrc audio, const float *__restrict__ window,
+                 EncSubStats *__restrict__ stats, double *__restrict__ autoc_out) {
+    // subframe g of this launch: frame g / nch, channel g % nch (channels [0, nch) of every frame)
+    __shared__ __align__(16) StatsWarpShared Sh[kStatsWarps];
+    const int lane = threadIdx.x & 31;
+    const uint32_t g = blockIdx.x * kStatsWarps + (threadIdx.x >> 5);
+    if (g >= total) return;
+    const uint32_t f = g / nch, ch = g - f * nch, task = f * channels + ch;
+    const TaskLoc L = locate_task(frames, audio, f, ch);
+    if (!fast_eligible(L)) return;
+    StatsWarpShared &S = Sh[threadIdx.x >> 5];
+    constexpr uint32_t n = kMaxBlock;
+    constexpr int HALO = NLAGS > 0 ? NLAGS - 1 : 0;
+    constexpr int NL = NLAGS > 0 ? NLAGS : 1;
+    const int32_t x_first = sample_at(L, 0);
+    uint32_t orv = 0, diff = 0, e32[5] = {0, 0, 0, 0, 0};
+    double r8 = 0.0, r1 = 0.0, r4 = 0.0;    // running totals of the root set: lag autoc_lag8(lane), lag 8, lag autoc_lag4(lane)
+#pragma unroll 1
+    for (int j = 0; j < 8; j++) {
+        const int t = 32 * j + lane;
+        int32_t xs[28];
+        load_samples28(L, t, xs);
+        float wv[kSPT + HALO + 1];
+        if constexpr (NLAGS > 0) load_window_chunk<HALO>(window, t, wv);
+        // fixed-predictor |residual| sums over all 16 samples (chunk 0's zero halo is corrected below); |4th difference|
+        // <= 16 * 2^15, so a lane's 128 samples and the warp's 4096 fit 32 bits
+        uint32_t c32[5] = {0, 0, 0, 0, 0};
+        int32_t d1[kSPT + 3], d2[kSPT + 2], d3[kSPT + 1];
+#pragma unroll
+        for (int k = 0; k < kSPT + 3; k++) d1[k] = xs[9 + k] - xs[8 + k];
+#pragma unroll
+        for (int k = 0; k < kSPT + 2; k++) d2[k] = d1[k + 1] - d1[k];
+#pragma unroll
+        for (int k = 0; k < kSPT + 1; k++) d3[k] = d2[k + 1] - d2[k];
+#pragma unroll
+        for (int s = 0; s < kSPT; s++) {
+            orv |= (uint32_t)xs[12 + s]; diff |= (uint32_t)(xs[12 + s] ^ x_first);
+            c32[0] = __sad(xs[12 + s], 0, c32[0]); c32[1] = __sad(xs[12 + s], xs[11 + s], c32[1]);
+            c32[2] = __sad(d1[s + 3], d1[s + 2], c32[2]); c32[3] = __sad(d2[s + 2], d2[s + 1], c32[3]);
+            c32[4] = __sad(d3[s + 1], d3[s], c32[4]);
+        }
+#pragma unroll
+        for (int q = 0; q < 5; q++) { S.ch[q][t] = c32[q]; e32[q] += c32[q]; }
+        if constexpr (NLAGS > 0) {
+            float df[kSPT + HALO];
+            window_full<HALO>(xs, wv, df);
+            double ac[NL];
+#pragma unroll
+            for (int l = 0; l < NLAGS; l++) ac[l] = 0.0;
+            autoc_fma<NLAGS>(df, ac);
+            double g8, g1, g4;
+            autoc_warp_sums<NLAGS>(ac, lane, g8, g1, g4);
+            r8 += g8; r1 += g1;
+            if (NLAGS > 9) r4 += g4;
+        }
+    }
+    orv = __reduce_or_sync(0xFFFFFFFFu, orv);
+    diff = __reduce_or_sync(0xFFFFFFFFu, diff);
+    uint32_t wasted = orv ? (uint32_t)(__ffs((int)orv) - 1) : 0;
+    if (wasted > bps_stream) wasted = bps_stream;
+    if (lane == 0) {
+        // chunk 0 summed its first 4 samples against a zero history: those terms are not part of the order guess's
+        // statistic (i in [4, n)), and the terms i < q are not part of the order-q residual
+        int32_t r[4] = {x_first, sample_at(L, 1), sample_at(L, 2), sample_at(L, 3)};
+#pragma unroll
+        for (int q = 0; q < 5; q++) {
+            uint32_t all = 0, pre = 0;
+#pragma unroll
+            for (int s = 0; s < 4; s++) { const uint32_t u = __sad(r[s], 0, 0u); all += u; if (s < q) pre += u; }
+            e32[q] -= all;
+            S.ch[q][0] -= pre;
+#pragma unroll
+            for (int s = 3; s >= 1; s--) r[s] -= r[s - 1];          // next order's residual, zero history
+        }
+    }
+    unsigned long long e[5];
+#pragma unroll
+    for (int q = 0; q < 5; q++) e[q] = __reduce_add_sync(0xFFFFFFFFu, e32[q]) >> wasted;
+    EncSubStats *st = stats + task;
+    if (lane < 5) st->e[lane] = lane == 0 ? e[0] : lane == 1 ? e[1] : lane == 2 ? e[2] : lane == 3 ? e[3] : e[4];
+    uint32_t flags = diff == 0 ? 1u : 0u;
+    if (diff != 0) {
+        // ---- FIXED candidate: libFLAC's order guess, its "worth trying" estimate and the Rice search (k_enc_fixed) ----
+        uint32_t guess;
+        const unsigned long long m1234 = min(min(e[1], e[2]), min(e[3], e[4]));
+        const unsigned long long m234 = min(e[2], min(e[3], e[4]));
+        const unsigned long long m34 = min(e[3], e[4]);
+        if (e[0] <= m1234) guess = 0; else if (e[1] <= m234) guess = 1; else if (e[2] <= m34) guess = 2; else if (e[3] <= e[4]) guess = 3; else guess = 4;
+        const uint32_t bps = bps_stream - wasted;
+        const unsigned long long eg = guess == 0 ? e[0] : guess == 1 ? e[1] : guess == 2 ? e[2] : guess == 3 ? e[3] : e[4];
+        if (!(fixed_bits_estimate(eg) >= (float)bps)) {
+            __syncwarp();
+            // lane l sums chunks [8l, 8l + 8) in two halves; finest partitions are 2^(8 - P) chunks
+            const uint4 u = *reinterpret_cast<const uint4 *>(&S.ch[guess][8 * lane]);
+            const uint4 v = *reinterpret_cast<const uint4 *>(&S.ch[guess][8 * lane + 4]);
+            const uint32_t a = (u.x + u.y + u.z + u.w) >> wasted, b = (v.x + v.y + v.z + v.w) >> wasted;
+            if (max_po_cfg == 6) { S.fin[2 * lane] = a; S.fin[2 * lane + 1] = b; }
+            else {
+                const uint32_t lg = 5 - max_po_cfg;                  // octets per finest partition: 2^0..2^2
+                uint32_t p = a + b;
+#pragma unroll
+                for (int step = 0; step < 2; step++)
+                    if ((uint32_t)step < lg) p += __shfl_xor_sync(0xFFFFFFFFu, p, 1 << step);
+                if (((uint32_t)lane & ((1u << lg) - 1u)) == 0) S.fin[(uint32_t)lane >> lg] = p;
+            }
+            __syncwarp();
+            uint32_t rb, best_l;
+            warp_search(S.fin, guess, max_po_cfg, bps_stream > 16 ? 31u : 15u, lane, st->fx_params, &rb, &best_l);
+            if (lane == 0) { st->fx_bits = 8 + wasted + guess * bps + rb; st->fx_po = max_po_cfg - best_l; }
+            flags |= 2u;
+        }
+        if (lane == 0) st->fx_order = guess;
+    }
+    if (lane == 0) { st->wasted = wasted; st->flags = flags; st->fx_bad = 0; }
+    if constexpr (NLAGS > 0) {
+        if (diff == 0) return;
+        const double sc = ldexp(1.0, -2 * (int)wasted);
+        double *out = autoc_out + (size_t)task * kMaxSets * kLags;
+        if ((lane & 3) == 0) out[autoc_lag8(lane)] = r8 * sc;
+        if (lane == 0) out[8] = r1 * sc;
+        if (NLAGS > 9 && (lane & 7) == 0) out[autoc_lag4(lane)] = r4 * sc;
+        // ---- subdivide_tukey sets: halves (b = 2), thirds (b = 3) ----
+        int set = 1;
+        for (uint32_t b = 2; b <= windows; b++) {
+            for (uint32_t sub = 0; sub < b; sub++, set++) {
+                const uint32_t part = n / b / 2, wshift = (sub * n) / b, wlen = n / b;
+                r8 = 0.0; r1 = 0.0; r4 = 0.0;
+#pragma unroll 1
+                for (int j = 0; j < 8; j++) {
+                    // a row of chunks wholly outside the window adds +0.0 to every running total (never -0.0): skipped
+                    if (!(512u * j + 512u > wshift && 512u * j < wshift + wlen)) continue;
+                    const int t = 32 * j + lane;
+                    const uint32_t i0 = (uint32_t)t * kSPT;
+                    double ac[NL];
+#pragma unroll
+                    for (int l = 0; l < NLAGS; l++) ac[l] = 0.0;
+                    if (i0 + kSPT > wshift && i0 < wshift + wlen) {
+                        int32_t xs[28];
+                        load_samples28(L, t, xs);
+                        if (wasted) {
+#pragma unroll
+                            for (int k = 0; k < 28; k++) xs[k] >>= wasted;
+                        }
+                        float df[kSPT + HALO];
+                        window_part<HALO>(xs, i0, wshift, wlen, part, window, df);
+                        autoc_fma<NLAGS>(df, ac);
+                    }
+                    double g8, g1, g4;
+                    autoc_warp_sums<NLAGS>(ac, lane, g8, g1, g4);
+                    r8 += g8; r1 += g1;
+                    if (NLAGS > 9) r4 += g4;
+                }
+                double *o = autoc_out + ((size_t)task * kMaxSets + set) * kLags;
+                if ((lane & 3) == 0) o[autoc_lag8(lane)] = r8;
+                if (lane == 0) o[8] = r1;
+                if (NLAGS > 9 && (lane & 7) == 0) o[autoc_lag4(lane)] = r4;
+            }
+        }
+    }
 }
 
 // ------------------------------------------------------------------------------------------------ model
